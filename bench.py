@@ -5,6 +5,7 @@ a non-zero exit).
 
   python bench.py --gpus N --steps K --warmup W            our arm: the CUDA path through the C ABI
   python bench.py --impl reference --gpus N ...            the reference's CPU path (oracle port), host threads
+  python bench.py ... --dump-outputs DIR                   also write what each timed leg returned in its last step
 
 A step = one pass of scan -> predicate -> MVCC -> aggregate over the batch, through llkv_gpu_agg_execute (fresh accumulators,
 one fused scan, merge of the ranks' partial states) and llkv_gpu_agg_finalize (result in host memory).
@@ -23,6 +24,8 @@ import sys
 import threading
 import time
 
+# the benchmark writes nothing into the source tree, which may be read-only
+sys.dont_write_bytecode = True
 # stdout carries exactly one JSON line: NCCL's own banner ("NCCL version ...") goes to stderr
 os.environ.setdefault("NCCL_DEBUG_FILE", "/dev/stderr")
 
@@ -294,14 +297,15 @@ def run_ours(args):
             step(True)
         barrier()
         dt = max_over_ranks(time.perf_counter() - t0)
-        merged = plain_rows(agg.decode(*raw))
+        rows = agg.decode(*raw)
+        merged = plain_rows(rows)
         check(merged == want_all, f"{name}: merged result {merged} != numpy over all shards {want_all}")
         info = agg.run_info()
         agg.destroy()
         prog.destroy()
         # the merge kernel's device time on every rank (it includes waiting for the slowest peer's scan)
         merge_all = gather(statistics.mean(merge_ms)) if merge_ms and world > 1 else None
-        return {"seconds": dt, "kernel_ms": kernel_ms, "merge_ms": merge_all, "launches": launches, "info": info, "result": merged}
+        return {"seconds": dt, "kernel_ms": kernel_ms, "merge_ms": merge_all, "launches": launches, "info": info, "result": merged, "rows": rows}
 
     failed = None
     sampler = ClockSampler(local)
@@ -334,7 +338,7 @@ def run_ours(args):
         for _ in range(max(1, min(args.warmup, 2))):
             e2e_step()
         barrier()
-        e2e_steps = max(1, min(args.steps, 5))
+        e2e_steps = args.steps
         moved0 = sum(dcs[f].h2d_bytes() for f in e2e_cols)
         t0 = time.perf_counter()
         for _ in range(e2e_steps):
@@ -347,11 +351,20 @@ def run_ours(args):
         agg.destroy()
         prog.destroy()
 
+        # --dump-outputs: the merged results are the same on every rank, rank 0 writes them
+        dump = {} if args.dump_outputs and rank == 0 else None
+        if dump is not None:
+            add_result(dump, "q6", q6["rows"])
+            if q1 is not None:
+                add_result(dump, "q1", q1["rows"])
+            add_result(dump, "e2e_q6", e2e_result)
         extra = {}
         if world == 1 and not args.no_configs:
-            extra["config0"] = bench_config0(ctx, gpu, args)
+            extra["config0"] = bench_config0(ctx, gpu, args, dump)
         if world == 1 and not args.no_highcard:
-            extra["highcard"] = bench_highcard(ctx, gpu, torch, args, big=n >= 20_000_000)
+            extra["highcard"] = bench_highcard(ctx, gpu, torch, args, big=n >= 20_000_000, dump=dump)
+        if dump is not None:
+            write_outputs(args.dump_outputs, dump)
         clocks = sampler.stop() if rank == 0 else None  # sampled across the timed regions
 
         total_rows = sum(gather_rows(dist, n, world))
@@ -454,6 +467,30 @@ def run_ours(args):
         sys.exit(1)
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+DUMP_GROUPS = 1 << 18  # groups of a high-cardinality result that --dump-outputs keeps
+
+
+def add_result(dump, name, rows):
+    """Decoded result rows as float64 arrays `<name>_values` [groups, aggregates] and, when grouped, `<name>_keys`
+    [groups, keys]: a Decimal128 as its value (unscaled / 10^scale), a one-character Utf8 key as its code point, NULL as NaN."""
+    def num(x, scale=0):
+        if x is None:
+            return float("nan")
+        return float(ord(x)) if isinstance(x, str) else x / 10 ** scale
+    dump[name + "_values"] = np.array([[num(v.value, v.scale) for v in vals] for _, vals in rows], dtype=np.float64)
+    if rows and rows[0][0]:
+        dump[name + "_keys"] = np.array([[num(k) for k in key] for key, _ in rows], dtype=np.float64)
+
+
+def write_outputs(directory, dump):
+    total = sum(a.nbytes for a in dump.values())
+    check(total <= DUMP_LIMIT_BYTES, f"--dump-outputs: {total} bytes, more than {DUMP_LIMIT_BYTES}")
+    os.makedirs(directory, exist_ok=True)
+    for name, a in dump.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def gather_rows(dist, n, world):
     if dist is None:
         return [n]
@@ -462,10 +499,10 @@ def gather_rows(dist, n, world):
     return out
 
 
-def bench_config0(ctx, gpu, args):
+def bench_config0(ctx, gpu, args, dump):
     """BASELINE.json configs[0]: SELECT SUM(x) FROM t WHERE x BETWEEN a AND b over one Int64 column of 10 M rows (a, b = 25th / 75th
     percentile), without and with the MVCC columns every SQL table carries.  Launch-latency bound at this size: the 1 B-row figure is
-    the Q6 / Q1 legs' business.  Results against numpy."""
+    the Q6 / Q1 legs' business.  Results against numpy; with `dump` (a dict), the last step's results are added to it."""
     n = 10_000_000
     t, snap = tpch.int64_table(n, seed=1, table_id=3)
     x = t.columns[tpch.X_FIELD].values
@@ -484,7 +521,7 @@ def bench_config0(ctx, gpu, args):
                 agg.execute(prog, sn is not None)
                 got = agg.finalize(1)
             torch_sync(ctx)
-            steps = max(args.steps, 20)
+            steps = args.steps
             t0 = time.perf_counter()
             for _ in range(steps):
                 agg.execute(prog, sn is not None)
@@ -494,6 +531,8 @@ def bench_config0(ctx, gpu, args):
             dtm = time.perf_counter() - t0
             got = agg.decode(*raw)
             check(got[0][1][0].value == want, f"configs[0] {name}: {got[0][1][0].value} != numpy {want}")
+            if dump is not None:
+                add_result(dump, f"config0_{name}", got)
             info = agg.run_info()
             kms = statistics.mean(ms)
             out[name] = {"value": n * steps / dtm, "ms_per_step": dtm / steps * 1e3, "kernel_ms": kms, "bytes_per_row": info.physical_bytes_per_row,
@@ -510,11 +549,12 @@ def torch_sync(ctx):
     ctx.synchronize()
 
 
-def bench_highcard(ctx, gpu, torch, args, big):
+def bench_highcard(ctx, gpu, torch, args, big, dump):
     """BASELINE.json configs[3]: GROUP BY over 10 M distinct Int64 keys, SUM + COUNT, 1 B rows (key = SplitMix64(i) mod 10^7,
     value = SplitMix64(i + 2^40) mod 1001).  The two columns are generated on the device in pieces (16 GB of input) and appended from
     device memory; kernel time only (CUDA events around the scan + apply launches).  Every group's SUM and COUNT is compared
-    with an integer scatter-add of the same arrays (torch, exact int64)."""
+    with an integer scatter-add of the same arrays (torch, exact int64).  With `dump` (a dict), a fixed sample of the last run's
+    groups is added to it."""
     rows, n_keys = (args.highcard_rows or 1_000_000_000, 10_000_000) if big else (1 << 22, 2_000_000)
     dev = torch.device("cuda", ctx.device)
     piece = 1 << 26
@@ -571,7 +611,7 @@ def bench_highcard(ctx, gpu, torch, args, big):
             ctx.set_partitioning(mode)
             hagg = gpu.Aggregation(dt, tpch.highcard_aggregates(), (tpch.K_FIELD,), cardinality_hint=n_keys)
             ms = []
-            for i in range(4):
+            for i in range(1 + args.steps):
                 hagg.reset()
                 hagg.run(None, False, 0, rows)
                 groups = hagg.group_count()
@@ -588,6 +628,12 @@ def bench_highcard(ctx, gpu, torch, args, big):
             check(int(torch.unique(kk).numel()) == n_groups, f"configs[3] {name}: duplicate keys in the result")
             order = first[kk]
             check(bool((order[1:] > order[:-1]).all().item()), f"configs[3] {name}: groups are not in first-appearance order")
+            if dump is not None:
+                # the same groups from run to run: a seeded choice of positions in key order
+                by_key = np.argsort(keys["bits"][:, 0].astype(np.int64), kind="stable")
+                pick = by_key[np.sort(np.random.default_rng(0).choice(n_groups, min(n_groups, DUMP_GROUPS), replace=False))]
+                dump[f"highcard_{name}_keys"] = keys["bits"][pick, :1].astype(np.int64).astype(np.float64)
+                dump[f"highcard_{name}_values"] = vals["lo"][pick].astype(np.int64).astype(np.float64)
             hagg.destroy()
             del kk, got_sum, got_cnt, order
             kms_hc = statistics.mean(ms)
@@ -723,7 +769,11 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-highcard", action="store_true")
     ap.add_argument("--no-configs", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what each timed leg returned in its last step as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3
     if args.impl == "reference":
