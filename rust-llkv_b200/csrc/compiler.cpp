@@ -2229,7 +2229,8 @@ class Emitter {
           if (!(x.lo > -lim && x.hi < lim)) return lf_fail(__LINE__);  // the precision check could turn a value into NULL
           if (st.back().where == Sym::LIT) { fold_lit(st.back(), x.lo); break; }
           load_acc(st.size() - 1);
-          femit(FO_DIVR, in.a, src.lo >= 0 ? (src.hi < ((i128)1 << 32) ? 2 : 1) : 0, 0);
+          // the 32-bit division needs the divisor in 32 bits too: 10^k for k <= 9
+          femit(FO_DIVR, in.a, src.lo >= 0 ? (src.hi < ((i128)1 << 32) && in.a <= 9 ? 2 : 1) : 0, 0);
           st.back().iv = x;
           break;
         }

@@ -101,7 +101,8 @@ enum FastOp : uint16_t {
   FO_OP_COL,      // acc = acc op column.     a = FastBin | FB_REV (column op acc), b = LoadKind, c = column
   FO_OP_LIT,      // acc = acc op literal.    a = FastBin | FB_REV, c = literal index
   FO_OP_TMP,      // acc = acc op tmp[b].     a = FastBin | FB_REV
-  FO_DIVR,        // a = k, b = 0 signed / 1 non-negative / 2 non-negative and < 2^32: acc / 10^k rounded half away from zero
+  FO_DIVR,        // a = k, b = 0 signed / 1 non-negative / 2 non-negative and < 2^32 with k <= 9 (value and divisor in 32
+                  // bits): acc / 10^k rounded half away from zero
   FO_MULP,        // a = k: acc * 10^k (proven not to overflow)
   FO_I2F,         // i64 -> f64
   FO_D2F,         // c = literal holding 10^scale as f64: (f64)acc / 10^scale
