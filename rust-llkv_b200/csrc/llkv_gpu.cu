@@ -658,12 +658,12 @@ struct llkv_gpu_ctx {
   bool timing = false;
   int tune_ctas = 0, tune_block = 0, tune_stages = 0, tune_rpt = 0, tune_force_wide = 0;
   int jit_mode = 1;  // 0 never, 1 specialise a plan shape from its second run on, 2 always
-  int partition_mode = 1;  // partitioned high-cardinality GROUP BY: 0 never, 1 when the table exceeds L2, 2 whenever possible
+  int partition_mode = 1;  // partitioned high-cardinality GROUP BY: 0 never, 1 when the table exceeds L2, 2 whenever possible,
+                           // 3 as 2 but never in packed tuples
   int prune_mode = 1;      // zone-map tile skipping: 0 never, 1 columns scanned again unchanged + >= 1/8 of the tiles, 2 always
   std::map<std::string, uint32_t> shape_runs;
   bool keep_wide_decimals = false;  // LLKV_GPU_KEEP_WIDE_DECIMALS=1: never narrow Decimal128 columns at seal
   bool no_d32 = false;              // LLKV_GPU_NO_D32=1: narrow to i64 only (experiments)
-  bool no_packed = false;           // LLKV_GPU_NO_PACKED=1: partitioned GROUP BY in its first form only (experiments)
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
   cudaEvent_t ev2 = nullptr, ev3 = nullptr;  // around the peer-mailbox merge kernel (timing)
   void* nccl_comm = nullptr;
@@ -820,6 +820,23 @@ struct PendingRun {
   bool timed_merge = false;
 };
 
+// The forms a lean plan runs in: the interpreting build, the build specialised on the plan shape, and the two partitioned
+// forms of a high-cardinality GROUP BY (specialised builds only) — multi-field tuples, and packed tuples
+enum LeanForm { LEAN_INTERPRETED, LEAN_SPECIALISED, LEAN_PARTITIONED, LEAN_PACKED, kLeanForms };
+struct LeanFormGeometry {
+  LeanPlan plan;
+  uint32_t grid = 0, ctas = 1;
+  bool have = false;
+};
+
+// Partition layout of the packed form.  Dense integer keys (the packed key range is within 4x the expected groups) make a
+// partition a key range whose shared-memory slots are indexed directly; otherwise partitions are ranges of the key's hash
+// with a small open-addressing table in shared memory (load factor <= 1/2 when the keys spread evenly).
+struct PackedLayout {
+  uint32_t parts = 0, shift = 0, slots = 0, dense = 0, key_bits = 0, row_bits = 0, n_ops = 0;
+  uint32_t op_bits[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+};
+
 struct llkv_gpu_agg {
   llkv_gpu_ctx* ctx = nullptr;
   StringStore strings;
@@ -855,12 +872,11 @@ struct llkv_gpu_agg {
   bool in_rerun = false;
   // the lean plan of the previous run, reusable while request_signature() does not change
   LeanPlan lean;
-  LeanPlan lean2[4];  // [0] interpreted geometry, [1] geometry of the specialised build, [2] specialised + partitioned, [3] + packed tuples
-  bool lean_have[4] = {false, false, false, false};
-  uint32_t lean_grid2[4] = {0, 0, 0, 0}, lean_ctas2[4] = {1, 1, 1, 1};
-  // packed form: partition layout of the current plan
-  uint32_t pk_parts = 0, pk_shift = 0, pk_slots = 0, pk_dense = 0, pk_key_bits = 0, pk_row_bits = 0, pk_n_ops = 0, pk_used_parts = 0;
-  uint32_t pk_op_bits[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  LeanFormGeometry forms[kLeanForms];  // the geometry of each form, computed when a run first asks for it
+  PackedLayout packed;                 // packed form: partition layout of the current plan
+  void forget_forms() {
+    for (LeanFormGeometry& f : forms) f.have = false;
+  }
   // partitioned high-cardinality GROUP BY: tuple partitions and their fill counters, kept across runs
   u64* part_out = nullptr;
   size_t part_out_elems = 0;
@@ -957,8 +973,6 @@ extern "C" int32_t llkv_gpu_ctx_create(int32_t device_ordinal, int32_t n_streams
     c->keep_wide_decimals = e && e[0] == '1';
     const char* e32 = getenv("LLKV_GPU_NO_D32");
     c->no_d32 = e32 && e32[0] == '1';
-    const char* ep = getenv("LLKV_GPU_NO_PACKED");
-    c->no_packed = ep && ep[0] == '1';
     const char* ed = getenv("LLKV_GPU_DMA_SHARE");  // percent (experiments)
     if (ed && ed[0]) c->dma_share = std::max(-1, std::min(100, atoi(ed)));
     const char* eg = getenv("LLKV_GPU_NO_GRAPHS");  // (profilers that want plain launches)
@@ -2795,35 +2809,31 @@ static u64 next_pow2(u64 v) {
   return p;
 }
 
-// Chooses block size, rows per thread, pipeline depth and CTA-local group slots so that the plan fits in shared memory,
-// and fills the launch-geometry / shared-memory fields of the plan.
-static int32_t plan_geometry(llkv_gpu_ctx* ctx, Plan& p, bool wide, bool fast, uint64_t row_begin, uint64_t row_end, uint64_t hint,
-                             Geometry& g) {
+// Rows of a grouped aggregate's global table at its first run: small when the caller knows the cardinality (Q1: 6 groups
+// -> 32 rows), since finalize and the multi-GPU merge move the whole table; it grows x4 on FLAG_TABLE_FULL if the hint was wrong
+static u64 group_table_cap(u64 hint) { return hint ? next_pow2(std::max<u64>(32, hint * 2)) : 1024; }
+
+// General interpreter: chooses block size, rows per thread, pipeline depth and CTA-local group slots so that the plan fits
+// in shared memory, and fills the launch-geometry / shared-memory fields of the plan.
+static int32_t plan_geometry(llkv_gpu_ctx* ctx, Plan& p, bool wide, uint64_t row_begin, uint64_t row_end, uint64_t hint, Geometry& g) {
   const uint32_t vbytes = wide ? 16u : 8u;
-  uint32_t NT = ctx->tune_block ? (uint32_t)ctx->tune_block : (fast ? 128u : 512u);
-  uint32_t R = ctx->tune_rpt ? (uint32_t)ctx->tune_rpt : (wide ? 1u : (fast ? 4u : 2u));
+  uint32_t NT = ctx->tune_block ? (uint32_t)ctx->tune_block : 512u;
+  uint32_t R = ctx->tune_rpt ? (uint32_t)ctx->tune_rpt : (wide ? 1u : 2u);
   if (wide && R > 2) R = 2;
-  if (!fast && R > 4) R = 4;
-  if (fast) {  // launch bounds of fast_scan_kernel<R>
-    const uint32_t cap = R >= 8 ? 128u : 256u;
-    if (NT > cap) NT = cap;
-  }
-  uint32_t stages = ctx->tune_stages ? (uint32_t)ctx->tune_stages : (fast ? 2u : 3u);
-  if (fast && stages < 2) stages = 2;  // the lean kernel is always staged
-  uint32_t ctas = ctx->tune_ctas ? (uint32_t)ctx->tune_ctas : (fast ? 4u : 2u);
+  if (R > 4) R = 4;
+  uint32_t stages = ctx->tune_stages ? (uint32_t)ctx->tune_stages : 3u;
+  uint32_t ctas = ctx->tune_ctas ? (uint32_t)ctx->tune_ctas : 2u;
   uint32_t FG = 0;
   if (p.n_fast_words) {
     if (p.n_keys == 0) FG = 1;
     else if (hint == 0) FG = 16;
     else if (hint <= 128) FG = (uint32_t)next_pow2(hint + hint / 2 + 1);
-    else FG = fast ? 32 : 0;  // high cardinality: the lean kernel still folds the hottest keys per CTA, the rest go global
   }
   const uint32_t budget_total = (uint32_t)ctx->max_smem;
   for (int attempt = 0; attempt < 64; ++attempt) {
     const uint32_t T = NT * R;
     const bool staged = stages >= 2;
     uint32_t off = align_up((uint32_t)sizeof(Plan), 128);
-    p.smem_plan_off = 0;
     p.smem_bar_off = off;
     off += 128;
     p.smem_stage_off = off;
@@ -2842,17 +2852,10 @@ static int32_t plan_geometry(llkv_gpu_ctx* ctx, Plan& p, bool wide, bool fast, u
       off += stage_bytes * stages;
     }
     p.smem_acc_off = off;
-    if (fast) {
-      off += align_up(FG * p.n_fast_words * (NT / 32) * 8, 128);  // one accumulator row per warp and group slot
-      p.smem_spill_off = off;
-      p.smem_tmp_off = off;
-      off += align_up(p.fast_tmps * T * 8, 128);  // tile-sized temporaries of the accumulator machine
-    } else {
-      off += align_up(FG * p.n_fast_words * NT * 8, 128);
-      p.smem_spill_off = off;
-      const uint32_t spill_slots = p.max_depth > 2 ? p.max_depth - 2 : 0;
-      off += align_up(spill_slots * R * NT * vbytes, 128);
-    }
+    off += align_up(FG * p.n_fast_words * NT * 8, 128);
+    p.smem_spill_off = off;
+    const uint32_t spill_slots = p.max_depth > 2 ? p.max_depth - 2 : 0;
+    off += align_up(spill_slots * R * NT * vbytes, 128);
     p.smem_tbl_off = off;
     off += align_up((FG ? FG : 1) * 8, 128);
     const uint32_t per_cta_budget = budget_total / ctas - 1024;
@@ -2883,8 +2886,8 @@ static int32_t plan_geometry(llkv_gpu_ctx* ctx, Plan& p, bool wide, bool fast, u
     else if (R > 1) R /= 2;
     else if (FG > 4 && p.n_keys) FG /= 2;
     else if (NT > 128) NT /= 2;
-    else if (FG > 0 && p.n_keys && !fast) FG = 0;
-    else if (stages >= 2 && !fast) stages = 1;
+    else if (FG > 0 && p.n_keys) FG = 0;
+    else if (stages >= 2) stages = 1;
     else break;
   }
   return set_error(LLKV_ERR_INVALID_ARGUMENT, "query state does not fit in shared memory on this path");
@@ -2899,8 +2902,7 @@ struct LeanTune {
                              // is amortised over the rows per thread, so rows per thread weigh more than resident warps
   bool partition = false;    // partitioned high-cardinality GROUP BY: the scan emits tuples (LeanTile::scatter)
   // packed form of it (LeanTile::scatter_packed): one 64-bit tuple per row, partitions aggregated in shared memory
-  bool packed = false;
-  uint32_t pack_key_bits = 0, pack_row_bits = 0, pack_parts = 0, pack_op_bits[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  const PackedLayout* packed = nullptr;
 };
 
 // The packed form needs: integer-packed keys narrower than 64 bits, after GROUP only COUNT / first row / SUMs whose
@@ -2947,13 +2949,7 @@ static bool partition_eligible(const Plan& p) {
   }
   return after_group && fields <= 2 + (uint32_t)kMaxPartOperands;
 }
-// Partition layout of the packed form.  Dense integer keys (the packed key range is within 4x the expected groups) make a
-// partition a key range whose shared-memory slots are indexed directly; otherwise partitions are ranges of the key's hash
-// with a small open-addressing table in shared memory (load factor <= 1/2 when the keys spread evenly).
-struct PackedLayout {
-  uint32_t parts = 0, shift = 0, slots = 0, dense = 0, key_bits = 0, row_bits = 0, n_ops = 0;
-  uint32_t op_bits[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-};
+// The packed form's partition layout; false when the plan or the hint rules the packed form out
 static bool packed_layout(const Plan& p, u64 hint, u64 gcap, bool small_tables, PackedLayout& L) {
   L = PackedLayout();
   if (!hint) return false;
@@ -2985,6 +2981,23 @@ static bool packed_layout(const Plan& p, u64 hint, u64 gcap, bool small_tables, 
   L.dense = dense ? 1u : 0u;
   return true;
 }
+
+// The form policy of a grouped lean plan, for the runtime and for llkv_gpu_debug_plan alike: LEAN_PACKED (layout in L),
+// LEAN_PARTITIONED, or LEAN_INTERPRETED when the plan keeps the per-row form.  Partitioning is worth two extra streaming
+// passes over the tuples once the group table is far larger than L2 (every row is then a random DRAM read-modify-write);
+// it needs the specialised kernel.  direct_global: that of the interpreted geometry (a hint above 128).
+static LeanForm partition_form(const Plan& p, int partition_mode, int jit_mode, bool direct_global, u64 hint, u64 gcap, u64 rows,
+                               PackedLayout& L) {
+  if (!partition_mode || !jit_mode || !direct_global || !partition_eligible(p) || gcap < 64) return LEAN_INTERPRETED;
+  const u64 table_bytes = gcap * (8ull + 8ull * p.n_gwords);
+  const bool big = table_bytes > (64ull << 20) && rows >= (4ull << 20);
+  if (!big && partition_mode < 2) return LEAN_INTERPRETED;
+  // Packed form first: one 64-bit tuple per row into partitions of a few thousand groups, each aggregated in shared memory
+  // by partition_fold_kernel.
+  if (partition_mode != 3 && packed_layout(p, hint, gcap, partition_mode == 2, L)) return LEAN_PACKED;
+  return LEAN_PARTITIONED;
+}
+
 static int32_t lean_geometry(const LeanTune& tn, const Plan& p, uint64_t row_begin, uint64_t row_end, uint64_t hint, LeanPlan& lp, Geometry& g,
                              uint32_t* ctas_out) {
   memset(&lp, 0, sizeof(lp));
@@ -3057,10 +3070,10 @@ static int32_t lean_geometry(const LeanTune& tn, const Plan& p, uint64_t row_beg
         if (lean_takes_operand(p.fcode[i].op)) ++s.n_fields;
       if (tn.packed) {
         s.partition = 2;
-        s.pack_key_bits = tn.pack_key_bits;
-        s.pack_row_bits = tn.pack_row_bits;
-        s.pack_parts = tn.pack_parts;
-        for (int j = 0; j < 8; ++j) s.pack_op_bits[j] = tn.pack_op_bits[j];
+        s.pack_key_bits = tn.packed->key_bits;
+        s.pack_row_bits = tn.packed->row_bits;
+        s.pack_parts = tn.packed->parts;
+        for (int j = 0; j < 8; ++j) s.pack_op_bits[j] = tn.packed->op_bits[j];
       }
     }
     while (FG > 4 && (u64)FG * thread_bytes * NC > 64u * 1024u) FG /= 2;
@@ -3365,22 +3378,21 @@ extern "C" int32_t llkv_gpu_debug_plan(const llkv_debug_column* cols, int32_t n_
     tn.rpt = rows_per_thread;
     tn.stages = stages;
     tn.ctas = ctas_per_sm;
-    tn.partition = (jit & 2) != 0 && partition_eligible(cr.plan);  // jit bit 1: the partitioned form of a GROUP BY
-    if (tn.partition && (jit & 8)) {  // jit bit 3: its packed form, when the plan allows it
-      PackedLayout L;
-      const u64 gcap = next_pow2(std::max<u64>(32, cardinality_hint * 2));
-      if (packed_layout(cr.plan, cardinality_hint, gcap, true, L)) {
-        tn.packed = true;
-        tn.pack_key_bits = L.key_bits;
-        tn.pack_row_bits = L.row_bits;
-        tn.pack_parts = L.parts;
-        for (int j = 0; j < 8; ++j) tn.pack_op_bits[j] = L.op_bits[j];
-      }
-    }
     LeanPlan lp;
     Geometry g;
     uint32_t ctas = 1;
     if ((rc = lean_geometry(tn, cr.plan, 0, rows, cardinality_hint, lp, g, &ctas))) return rc;
+    // jit bit 1: the partitioned form of a GROUP BY where the runtime would take it under partitioning mode 3; with bit 3,
+    // under mode 2 (packed tuples when the plan allows them).  The listing describes the specialised form whether or not
+    // bit 0 asks for its cubin.
+    PackedLayout L;
+    const int partition_mode = !(jit & 2) ? 0 : (jit & 8) ? 2 : 3;
+    const LeanForm form = partition_form(cr.plan, partition_mode, 1, lp.s.direct_global, cardinality_hint, group_table_cap(cardinality_hint), rows, L);
+    if (form != LEAN_INTERPRETED) {
+      tn.partition = true;
+      if (form == LEAN_PACKED) tn.packed = &L;
+      if ((rc = lean_geometry(tn, cr.plan, 0, rows, cardinality_hint, lp, g, &ctas))) return rc;
+    }
     lp.s.use_tile_list = (jit & 4) ? 1u : 0u;  // jit bit 2: the variant that walks a zone-map tile list
     text = lean_listing(lp, g, ctas);
     if (jit & 1) {
@@ -3439,7 +3451,7 @@ extern "C" int32_t llkv_gpu_filter_bitmap(llkv_gpu_ctx* ctx, uint64_t table_id, 
     CompileResult cr;
     if ((rc = compile_plan(req, cr))) { result = set_error(rc, "%s", cr.error.c_str()); break; }
     Geometry g;
-    if ((rc = plan_geometry(ctx, cr.plan, cr.wide, false, row_begin, row_end, 0, g))) { result = rc; break; }
+    if ((rc = plan_geometry(ctx, cr.plan, cr.wide, row_begin, row_end, 0, g))) { result = rc; break; }
     cr.plan.exists_bits = exists_bits;
     cr.plan.out_bitmap = d_bits;
     cr.plan.out_count = d_bits + alloc_words;
@@ -3613,13 +3625,7 @@ static int32_t agg_freeze_layout(llkv_gpu_agg* a, const CompileResult& cr) {
   a->gclass.assign(p.gword_class, p.gword_class + p.n_gwords);
   CUDA_TRY(cudaMalloc((void**)&a->d_gclass, a->n_gwords ? a->n_gwords : 1));
   CUDA_TRY(cudaMemcpy(a->d_gclass, a->gclass.data(), a->n_gwords, cudaMemcpyHostToDevice));
-  u64 gcap = 1;
-  if (p.n_keys) {
-    // a small table when the caller knows the cardinality (Q1: 6 groups -> 32 rows): finalize and the multi-GPU merge
-    // move the whole table; it grows x4 on FLAG_TABLE_FULL if the hint was wrong
-    gcap = a->hint ? next_pow2(std::max<u64>(32, a->hint * 2)) : 1024;
-  }
-  int32_t rc = agg_alloc_table(a, gcap);
+  int32_t rc = agg_alloc_table(a, p.n_keys ? group_table_cap(a->hint) : 1);
   if (rc) return rc;
   a->frozen = true;
   return LLKV_OK;
@@ -3898,150 +3904,111 @@ static int32_t agg_queue_result_copy(llkv_gpu_agg* a) {
   return LLKV_OK;
 }
 
-static int32_t agg_launch(llkv_gpu_agg* a, const llkv_gpu_program* prog, int apply_mvcc, uint64_t row_begin, uint64_t row_end,
-                          bool force_wide) {
-  llkv_gpu_ctx* ctx = a->ctx;
-  CompileRequest req;
-  std::vector<llkv_gpu_column*> handles;
-  uint64_t table_rows = 0;
-  int32_t rc = build_request(ctx, a->table_id, prog, apply_mvcc, req, handles, &table_rows);
-  if (rc) return rc;
-  if (row_end > table_rows) return set_error(LLKV_ERR_INVALID_ARGUMENT, "row_end %llu beyond the table's %llu rows", (unsigned long long)row_end, (unsigned long long)table_rows);
-  // Multi-GPU GROUP BY: the packed key layout (bits, minimum, string length per key) comes from column statistics, and
-  // partial tables can only be merged key by key if every rank packs alike.  The ranks agree on the statistics of the
-  // key columns (min of minima, max of maxima / string lengths) with one small all-reduce before compiling.
-  if (ctx->nccl_comm && ctx->n_ranks > 1 && !a->keys.empty()) {
-    bool changed = false;
-    if ((rc = agree_dictionaries(ctx, a, handles, &changed))) return rc;
-    if (changed) {  // columns were re-coded: their descriptions again
-      req = CompileRequest();
-      handles.clear();
-      if ((rc = build_request(ctx, a->table_id, prog, apply_mvcc, req, handles, &table_rows))) return rc;
-    }
-    if ((rc = agree_key_stats(ctx, a, req))) return rc;
-  }
-  Plan& p = a->cr.plan;
+// What agg_launch settles for one run before its launch loop
+struct RunLaunches {
   Geometry g;
-  LeanPlan& lean = a->lean;
   uint32_t lean_ctas = 1;
   bool use_jit = false;
-  const unsigned char* exists_bits = nullptr;
-  if ((rc = table_exists_bits(ctx, a->table_id, handles, table_rows, &exists_bits))) return rc;
-  const uint64_t sig = request_signature(ctx, req, prog, force_wide, exists_bits);
-  if (!(a->lean_sig == sig && a->cr.fast && a->frozen)) {
-    a->lean_sig = 0;
-    a->lean_jit_runs = 0;
-    a->lean_have[0] = a->lean_have[1] = a->lean_have[2] = a->lean_have[3] = false;
-    req.specs = a->specs.data();
-    req.n_aggs = (int32_t)a->specs.size();
-    req.agg_nodes = a->nodes.data();
-    req.n_agg_nodes = (int32_t)a->nodes.size();
-    req.key_fields = a->keys;
-    req.expr_mode = a->expr_mode;
-    req.force_wide = force_wide || ctx->tune_force_wide == 1;
-    req.no_fast = ctx->tune_force_wide != 0;
-    if ((rc = compile_plan(req, a->cr))) return set_error(rc, "%s", a->cr.error.c_str());
-    if ((rc = agg_freeze_layout(a, a->cr))) return rc;
-    p.exists_bits = exists_bits;
-    if (a->cr.fast) a->lean_sig = sig;
-    else if ((rc = plan_geometry(ctx, p, a->cr.wide, false, row_begin, row_end, a->hint, g))) return rc;
-  }
-  p.exists_bits = exists_bits;
-  if (a->cr.fast) {
-    // Two geometries per plan (kept while request_signature() does not change): [0] for the interpreting build (rows per
-    // thread first), [1] for a build specialised on the plan shape (resident warps first).  A shape is specialised once
-    // it repeats (jit_mode 1), always (2) or never (0); runs are counted on the interpreted shape.
-    auto geometry = [&](int which) -> int32_t {
-      if (a->lean_have[which]) return LLKV_OK;
-      LeanTune tn = lean_tune(ctx);
-      tn.interpreted = which == 0;
-      tn.partition = which >= 2;
-      if (which == 3) {
-        tn.packed = true;
-        tn.pack_key_bits = a->pk_key_bits;
-        tn.pack_row_bits = a->pk_row_bits;
-        tn.pack_parts = a->pk_parts;
-        for (int j = 0; j < 8; ++j) tn.pack_op_bits[j] = a->pk_op_bits[j];
-      }
-      Geometry gg;
-      uint32_t cc = 1;
-      // (a hint below the number of groups already seen would leave groups without a CTA-local slot: every row of such a
-      // group is a contended atomic on the global table)
-      const uint64_t hint_eff = a->hint && a->observed_groups > a->hint ? a->observed_groups : a->hint;
-      int32_t grc = lean_geometry(tn, p, row_begin, row_end, hint_eff, a->lean2[which], gg, &cc);
-      if (grc) return grc;
-      a->lean_grid2[which] = gg.grid;
-      a->lean_ctas2[which] = cc;
-      a->lean_have[which] = true;
-      return LLKV_OK;
-    };
-    if ((rc = geometry(0))) return rc;
-    if (ctx->jit_mode == 2) use_jit = true;
-    else if (ctx->jit_mode == 1) {
-      if (a->lean_jit_runs < 2) {
-        const std::string key(reinterpret_cast<const char*>(&a->lean2[0].s), sizeof(LeanShape));
-        a->lean_jit_runs = ++ctx->shape_runs[key];
-      }
-      use_jit = a->lean_jit_runs >= 2;
+  u64 max_rows = 0;    // rows per launch
+  PartPlan pp;         // partitioned form: the partition_apply pass behind every scan launch
+  FoldPlan fp;         // packed form: the partition_fold pass behind every scan launch
+  uint32_t part_grid = 0;
+  bool use_tile_list = false;
+};
+
+// Compiles the request and freezes the accumulator layout, unless the lean plan of the previous run still applies
+// (request_signature() unchanged).  A plan for the general interpreter gets its geometry here.
+static int32_t agg_compile(llkv_gpu_agg* a, CompileRequest& req, uint64_t sig, bool force_wide, uint64_t row_begin, uint64_t row_end,
+                           Geometry& g) {
+  llkv_gpu_ctx* ctx = a->ctx;
+  if (a->lean_sig == sig && a->cr.fast && a->frozen) return LLKV_OK;
+  a->lean_sig = 0;
+  a->lean_jit_runs = 0;
+  a->forget_forms();
+  req.specs = a->specs.data();
+  req.n_aggs = (int32_t)a->specs.size();
+  req.agg_nodes = a->nodes.data();
+  req.n_agg_nodes = (int32_t)a->nodes.size();
+  req.key_fields = a->keys;
+  req.expr_mode = a->expr_mode;
+  req.force_wide = force_wide || ctx->tune_force_wide == 1;
+  req.no_fast = ctx->tune_force_wide != 0;
+  int32_t rc;
+  if ((rc = compile_plan(req, a->cr))) return set_error(rc, "%s", a->cr.error.c_str());
+  if ((rc = agg_freeze_layout(a, a->cr))) return rc;
+  if (a->cr.fast) a->lean_sig = sig;
+  else if ((rc = plan_geometry(ctx, a->cr.plan, a->cr.wide, row_begin, row_end, a->hint, g))) return rc;
+  return LLKV_OK;
+}
+
+// The geometry of one form of the current lean plan, computed the first time a run asks for it
+static int32_t agg_form_geometry(llkv_gpu_agg* a, LeanForm form, uint64_t row_begin, uint64_t row_end) {
+  LeanFormGeometry& f = a->forms[form];
+  if (f.have) return LLKV_OK;
+  LeanTune tn = lean_tune(a->ctx);
+  tn.interpreted = form == LEAN_INTERPRETED;
+  tn.partition = form >= LEAN_PARTITIONED;
+  if (form == LEAN_PACKED) tn.packed = &a->packed;
+  Geometry g;
+  // (a hint below the number of groups already seen would leave groups without a CTA-local slot: every row of such a
+  // group is a contended atomic on the global table)
+  const uint64_t hint_eff = a->hint && a->observed_groups > a->hint ? a->observed_groups : a->hint;
+  int32_t rc = lean_geometry(tn, a->cr.plan, row_begin, row_end, hint_eff, f.plan, g, &f.ctas);
+  if (rc) return rc;
+  f.grid = g.grid;
+  f.have = true;
+  return LLKV_OK;
+}
+
+// Chooses the form the lean plan runs in and leaves it in a->lean.  A shape is specialised once it repeats (jit_mode 1),
+// always (2) or never (0); runs are counted on the interpreted shape.  A partitioned form (partition_form) is taken when its
+// specialised kernel is ready, the packed one first.
+static int32_t agg_choose_form(llkv_gpu_agg* a, uint64_t row_begin, uint64_t row_end, RunLaunches& r) {
+  llkv_gpu_ctx* ctx = a->ctx;
+  int32_t rc;
+  if ((rc = agg_form_geometry(a, LEAN_INTERPRETED, row_begin, row_end))) return rc;
+  if (ctx->jit_mode == 2) r.use_jit = true;
+  else if (ctx->jit_mode == 1) {
+    if (a->lean_jit_runs < 2) {
+      const std::string key(reinterpret_cast<const char*>(&a->forms[LEAN_INTERPRETED].plan.s), sizeof(LeanShape));
+      a->lean_jit_runs = ++ctx->shape_runs[key];
     }
-    int which = use_jit ? 1 : 0;
-    // Partitioned form of a high-cardinality GROUP BY: worth two extra streaming passes over the tuples once the group
-    // table is far larger than L2 (every row is then a random DRAM read-modify-write).  Needs the specialised kernel.
-    if (ctx->partition_mode && ctx->jit_mode && a->lean2[0].s.direct_global && partition_eligible(p)) {
-      const u64 table_bytes = a->gcap * (8ull + 8ull * a->n_gwords);
-      const bool big = table_bytes > (64ull << 20) && row_end - row_begin >= (4ull << 20);
-      if ((big || ctx->partition_mode >= 2) && a->gcap >= 64) {
-        // Packed form first: one 64-bit tuple per row into partitions of a few thousand groups, each aggregated in shared
-        // memory by partition_fold_kernel.  Dense integer keys (the key range is within 4x the expected groups) make a
-        // partition a key range whose slots are indexed directly; otherwise partitions are hash ranges with a small
-        // open-addressing table in shared memory.
-        PackedLayout L;
-        bool packed = false;
-        if (!ctx->no_packed && ctx->partition_mode != 3 && packed_layout(p, a->hint, a->gcap, ctx->partition_mode == 2, L)) {
-          if (a->pk_parts != L.parts || a->pk_shift != L.shift || a->pk_slots != L.slots || a->pk_dense != L.dense || a->pk_key_bits != L.key_bits ||
-              a->pk_row_bits != L.row_bits || a->pk_n_ops != L.n_ops || memcmp(a->pk_op_bits, L.op_bits, sizeof(L.op_bits)) != 0)
-            a->lean_have[3] = false;
-          a->pk_parts = L.parts;
-          a->pk_shift = L.shift;
-          a->pk_slots = L.slots;
-          a->pk_dense = L.dense;
-          a->pk_key_bits = L.key_bits;
-          a->pk_row_bits = L.row_bits;
-          a->pk_n_ops = L.n_ops;
-          memcpy(a->pk_op_bits, L.op_bits, sizeof(L.op_bits));
-          if ((rc = geometry(3)) == LLKV_OK && jit_ready(ctx->device, a->lean2[3], (int)a->lean_ctas2[3])) {
-            which = 3;
-            use_jit = true;
-            packed = true;
-          }
-        }
-        if (!packed) {
-          if ((rc = geometry(2))) return rc;
-          if (jit_ready(ctx->device, a->lean2[2], (int)a->lean_ctas2[2])) {
-            which = 2;
-            use_jit = true;
-          }
-        }
-      }
-    }
-    if ((rc = geometry(which))) return rc;
-    lean = a->lean2[which];
-    lean_ctas = a->lean_ctas2[which];
-    g.grid = a->lean_grid2[which];
-    g.block = lean.s.nc;
-    g.R = lean.s.rows_per_thread;
-    g.smem = lean.s.smem_total;
-    const uint32_t T = lean.s.tile_rows;
-    lean.row_begin = row_begin;
-    lean.row_end = row_end;
-    lean.first_tile = row_begin / T;
-    lean.n_tiles = row_end > row_begin ? (row_end + T - 1) / T - lean.first_tile : 0;
-    p.tile_rows = lean.s.tile_rows;
-    p.stages = lean.s.stages;
-    p.fast_groups = lean.s.fg;
+    r.use_jit = a->lean_jit_runs >= 2;
   }
-  // first-row words hold row ids (position + the row id of position 0), so shards of one table uploaded with their own
-  // row_id_base merge into the table's first-appearance order
+  LeanForm form = r.use_jit ? LEAN_SPECIALISED : LEAN_INTERPRETED;
+  PackedLayout L;
+  const LeanForm part = partition_form(a->cr.plan, ctx->partition_mode, ctx->jit_mode, a->forms[LEAN_INTERPRETED].plan.s.direct_global,
+                                       a->hint, a->gcap, row_end - row_begin, L);
+  auto ready = [&](LeanForm f) { return jit_ready(ctx->device, a->forms[f].plan, (int)a->forms[f].ctas); };
+  if (part == LEAN_PACKED) {
+    if (memcmp(&a->packed, &L, sizeof(L)) != 0) a->forms[LEAN_PACKED].have = false;
+    a->packed = L;
+    if (agg_form_geometry(a, LEAN_PACKED, row_begin, row_end) == LLKV_OK && ready(LEAN_PACKED)) form = LEAN_PACKED;
+  }
+  if (part != LEAN_INTERPRETED && form != LEAN_PACKED) {
+    if ((rc = agg_form_geometry(a, LEAN_PARTITIONED, row_begin, row_end))) return rc;
+    if (ready(LEAN_PARTITIONED)) form = LEAN_PARTITIONED;
+  }
+  if (form >= LEAN_PARTITIONED) r.use_jit = true;
+  if ((rc = agg_form_geometry(a, form, row_begin, row_end))) return rc;
+  const LeanFormGeometry& f = a->forms[form];
+  LeanPlan& lean = a->lean;
+  lean = f.plan;
+  r.lean_ctas = f.ctas;
+  r.g.grid = f.grid;
+  r.g.block = lean.s.nc;
+  r.g.R = lean.s.rows_per_thread;
+  r.g.smem = lean.s.smem_total;
+  Plan& p = a->cr.plan;
+  p.tile_rows = lean.s.tile_rows;
+  p.stages = lean.s.stages;
+  p.fast_groups = lean.s.fg;
+  return LLKV_OK;
+}
+
+// Points the run's plan at the aggregate's table and status word.  First-row words hold row ids (position + the row id of
+// position 0), so shards of one table uploaded with their own row_id_base merge into the table's first-appearance order.
+static int32_t agg_bind_state(llkv_gpu_agg* a, const std::vector<llkv_gpu_column*>& handles) {
   uint64_t row_origin = 0;
   for (size_t i = 0; i < handles.size(); ++i) {
     if (!handles[i]->has_origin) continue;
@@ -4050,6 +4017,8 @@ static int32_t agg_launch(llkv_gpu_agg* a, const llkv_gpu_program* prog, int app
                        (unsigned long long)handles[i]->row_id_origin, (unsigned long long)handles[0]->row_id_origin);
     row_origin = handles[i]->row_id_origin;
   }
+  Plan& p = a->cr.plan;
+  LeanPlan& lean = a->lean;
   p.row_origin = row_origin;
   lean.row_origin = row_origin;
   p.gkeys = a->gkeys;
@@ -4060,97 +4029,140 @@ static int32_t agg_launch(llkv_gpu_agg* a, const llkv_gpu_program* prog, int app
   lean.gwords = a->gwords;
   lean.gcap = a->gcap;
   lean.flags = a->d_flags;
-  const bool need_backup = a->cr.can_narrow_fail || p.n_keys != 0;
-  if (need_backup && (rc = agg_backup(a))) return rc;
-  a->pending.has_backup = need_backup;
-  // thread-private partial sums stay exact while a thread folds a bounded number of rows per launch: split very long scans
-  // (general interpreter: < 2^15 rows per thread; lean kernel: 2^kLeanRowsPerThreadLog2 rows per consumer thread, and
-  // launch-relative row indices must fit 32 bits)
-  const u64 threads = (u64)g.grid * g.block;
-  u64 max_rows_per_launch = threads * 32000ull;
-  if (a->cr.fast) max_rows_per_launch = std::min<u64>(max_rows_per_launch, 0xf0000000ull) / p.tile_rows * p.tile_rows;
-  // Partitioned GROUP BY: 2^bits partitions, each a contiguous slice of the table of about 24 MB (keys + words) so a
-  // slice and the tuple stream share L2 comfortably; a launch covers at most 2^28 rows so the tuple buffers stay bounded
-  // (capacity = the uniform share + 25 %; a partition that fills up — skewed keys — hands its surplus rows to the per-row
-  // path inside the scan, so no rerun is ever needed).
-  PartPlan pp;
-  FoldPlan fp;
-  uint32_t part_grid = 0;
-  const bool packed = a->cr.fast && lean.s.partition == 2;
-  const bool partitioned = a->cr.fast && lean.s.partition != 0;
-  if (packed) {
+  return LLKV_OK;
+}
+
+// The tuple partitions of a partitioned scan, in either form: sizes the launches (max_rows), and the capacity of a partition
+// as the uniform share of a launch's rows over `share` partitions + 25 %, of which `words` x part_cap fill part_out.
+// batch_rows: the longest launch.  LLKV_GPU_PART_BATCH_ROWS (tests: several launches on small tables) caps it when
+// env_caps, else replaces it.
+static int32_t agg_part_buffers(llkv_gpu_agg* a, u64 batch_rows, bool env_caps, u64 share, u64 words, u64 rows, u64& max_rows) {
+  const u64 T = a->cr.plan.tile_rows;
+  if (const char* e = getenv("LLKV_GPU_PART_BATCH_ROWS")) {
+    const u64 v = std::max<u64>(T, strtoull(e, nullptr, 10));
+    batch_rows = env_caps ? std::min<u64>(batch_rows, v) : v;
+  }
+  const u64 dense_max_rows = max_rows;
+  u64 part_cap = 0;
+  for (;;) {  // the tuple buffer of one launch; when HBM is short the launches get smaller instead
+    max_rows = std::max<u64>(T, std::min<u64>(dense_max_rows, batch_rows) / T * T);
+    const u64 launch_rows = std::min<u64>(rows + T, max_rows);
+    part_cap = (launch_rows / share + launch_rows / (4 * share) + 1024 + 15) / 16 * 16;
+    const size_t elems = (size_t)(words * part_cap);
+    if (a->part_out_elems >= elems) break;
+    if (a->part_out) CUDA_TRY(cudaFree(a->part_out));
+    a->part_out = nullptr;
+    a->part_out_elems = 0;
+    if (cudaMalloc((void**)&a->part_out, elems * 8) == cudaSuccess) {
+      a->part_out_elems = elems;
+      break;
+    }
+    cudaGetLastError();
+    a->part_out = nullptr;
+    if (batch_rows <= (1ull << 22)) return set_error(LLKV_ERR_IO, "out of device memory for the tuple partitions of a GROUP BY (%zu bytes)", elems * 8);
+    batch_rows >>= 1;
+  }
+  if (!a->part_cursor) CUDA_TRY(cudaMalloc((void**)&a->part_cursor, kMaxPackedPartitions * 4));
+  a->lean.part_out = a->part_out;
+  a->lean.part_cursor = a->part_cursor;
+  a->lean.part_cap = part_cap;
+  return LLKV_OK;
+}
+
+// The fold pass of the packed form
+static FoldPlan fold_plan(const llkv_gpu_agg* a) {
+  const LeanPlan& lean = a->lean;
+  FoldPlan fp{};
+  fp.tuples = a->part_out;
+  fp.cursor = a->part_cursor;
+  fp.part_cap = lean.part_cap;
+  fp.gkeys = a->gkeys;
+  fp.gwords = a->gwords;
+  fp.gcap = a->gcap;
+  fp.flags = a->d_flags;
+  fp.n_parts = a->packed.parts;
+  fp.n_gwords = lean.s.n_gwords;
+  fp.n_keys = lean.s.n_keys;
+  fp.key_bits = a->packed.key_bits;
+  fp.row_bits = a->packed.row_bits;
+  fp.dense = a->packed.dense;
+  fp.part_shift = a->packed.shift;
+  fp.slots = a->packed.slots;
+  fp.first_gword = ~0u;
+  for (uint32_t i = 0; i < lean.s.n_code; ++i) {  // operands in the order of the aggregates (lean_field_index)
+    const FInstr& in = lean.s.code[i];
+    if (in.op == FO_COUNT_STAR || in.op == FO_COUNT) fp.count_gword[fp.n_counts++] = in.c;
+    else if (in.op == FO_FIRSTROW) fp.first_gword = in.c;
+    else if (in.op == FO_SUM) {
+      fp.op_bits[fp.n_ops] = in.g;
+      fp.op_gword[fp.n_ops] = in.c;
+      fp.op_wide[fp.n_ops] = (in.a & 0x80) ? 1u : 0u;
+      ++fp.n_ops;
+    }
+  }
+  return fp;
+}
+
+// The apply pass of the partitioned form (multi-field tuples)
+static PartPlan part_plan(const llkv_gpu_agg* a, uint32_t n_parts) {
+  const LeanPlan& lean = a->lean;
+  PartPlan pp{};
+  pp.tuples = a->part_out;
+  pp.cursor = a->part_cursor;
+  pp.part_cap = lean.part_cap;
+  pp.gkeys = a->gkeys;
+  pp.gwords = a->gwords;
+  pp.gcap = a->gcap;
+  pp.flags = a->d_flags;
+  pp.n_parts = n_parts;
+  pp.n_fields = lean.s.n_fields;
+  pp.n_keys = lean.s.n_keys;
+  pp.n_gwords = lean.s.n_gwords;
+  pp.chunk = 2048;
+  pp.chunks_per_part = (uint32_t)((lean.part_cap + pp.chunk - 1) / pp.chunk);
+  for (uint32_t i = 0; i < lean.s.n_code; ++i) {  // operand fields follow the order of the aggregates (lean_field_index)
+    const FInstr& in = lean.s.code[i];
+    if (in.op < FO_COUNT_STAR || in.op > FO_FIRSTNAN) continue;
+    PartOp& o = lean_takes_operand(in.op) ? pp.vops[pp.n_vops++] : pp.nops[pp.n_nops++];
+    o.op = in.op;
+    o.flags = in.a;
+    o.gword = in.c;
+  }
+  return pp;
+}
+
+// Partitioned GROUP BY: the tuple partitions and the second pass of the chosen form.  Packed tuples go to partitions of a
+// few thousand groups (PackedLayout).  Multi-field tuples go to 2^bits hash partitions, each a contiguous slice of the table
+// of about 24 MB (keys + words) so a slice and the tuple stream share L2 comfortably.  A launch covers at most 2^28 rows
+// so the tuple buffers stay bounded; a partition that fills up (skewed keys) hands its surplus rows to the per-row path
+// inside the scan, so no rerun is ever needed.
+static int32_t agg_partitions(llkv_gpu_agg* a, const CompileRequest& req, uint64_t row_begin, uint64_t row_end, RunLaunches& r) {
+  llkv_gpu_ctx* ctx = a->ctx;
+  const Plan& p = a->cr.plan;
+  LeanPlan& lean = a->lean;
+  const uint32_t partition = a->cr.fast ? lean.s.partition : 0;
+  a->info.partitions = 0;
+  a->info.packed_tuples = 0;
+  int32_t rc;
+  if (partition == 2) {
     // partitions that can hold keys: all of them for hash ranges; for key ranges those below the largest packed key
-    u64 used = a->pk_parts;
-    if (a->pk_dense && p.n_keys == 1 && p.key_kind[0] == KK_INT) {
+    u64 used = a->packed.parts;
+    if (a->packed.dense && p.n_keys == 1 && p.key_kind[0] == KK_INT) {
       for (const ColumnMeta& c : req.cols)
         if (c.field_id == a->keys[0] && c.has_minmax) {
           const u64 kmax = c.max_bits - c.min_bits;  // (two's complement difference: also right for signed columns)
-          used = std::min<u64>(used, (kmax >> a->pk_shift) + 1);
+          used = std::min<u64>(used, (kmax >> a->packed.shift) + 1);
         }
     }
-    a->pk_used_parts = (uint32_t)used;
-    const u64 P = a->pk_parts;
-    u64 batch_rows = 1ull << a->pk_row_bits;
-    if (const char* e = getenv("LLKV_GPU_PART_BATCH_ROWS")) batch_rows = std::min<u64>(batch_rows, std::max<u64>(p.tile_rows, strtoull(e, nullptr, 10)));
-    const u64 dense_max_rows = max_rows_per_launch;
-    u64 part_cap = 0;
-    for (;;) {  // the tuple buffer of one launch; when HBM is short the launches get smaller instead
-      max_rows_per_launch = std::max<u64>(p.tile_rows, std::min<u64>(dense_max_rows, batch_rows) / p.tile_rows * p.tile_rows);
-      const u64 launch_rows = std::min<u64>(row_end - row_begin + p.tile_rows, max_rows_per_launch);
-      part_cap = (launch_rows / used + launch_rows / (4 * used) + 1024 + 15) / 16 * 16;
-      const size_t elems = (size_t)(P * part_cap);
-      if (a->part_out_elems >= elems) break;
-      if (a->part_out) CUDA_TRY(cudaFree(a->part_out));
-      a->part_out = nullptr;
-      a->part_out_elems = 0;
-      if (cudaMalloc((void**)&a->part_out, elems * 8) == cudaSuccess) {
-        a->part_out_elems = elems;
-        break;
-      }
-      cudaGetLastError();
-      a->part_out = nullptr;
-      if (batch_rows <= (1ull << 22)) return set_error(LLKV_ERR_IO, "out of device memory for the tuple partitions of a GROUP BY (%zu bytes)", elems * 8);
-      batch_rows >>= 1;
-    }
-    if (!a->part_cursor) CUDA_TRY(cudaMalloc((void**)&a->part_cursor, kMaxPackedPartitions * 4));
-    lean.part_out = a->part_out;
-    lean.part_cursor = a->part_cursor;
-    lean.part_cap = part_cap;
+    if ((rc = agg_part_buffers(a, 1ull << a->packed.row_bits, true, used, a->packed.parts, row_end - row_begin, r.max_rows))) return rc;
     lean.part_bits = 0;
-    lean.part_shift = a->pk_shift;
-    lean.part_dense = a->pk_dense;
-    memset(&fp, 0, sizeof(fp));
-    fp.tuples = a->part_out;
-    fp.cursor = a->part_cursor;
-    fp.part_cap = part_cap;
-    fp.gkeys = a->gkeys;
-    fp.gwords = a->gwords;
-    fp.gcap = a->gcap;
-    fp.flags = a->d_flags;
-    fp.n_parts = (uint32_t)P;
-    fp.n_gwords = lean.s.n_gwords;
-    fp.n_keys = lean.s.n_keys;
-    fp.key_bits = a->pk_key_bits;
-    fp.row_bits = a->pk_row_bits;
-    fp.dense = a->pk_dense;
-    fp.part_shift = a->pk_shift;
-    fp.slots = a->pk_slots;
-    fp.first_gword = ~0u;
-    for (uint32_t i = 0; i < lean.s.n_code; ++i) {  // operands in the order of the aggregates (lean_field_index)
-      const FInstr& in = lean.s.code[i];
-      if (in.op == FO_COUNT_STAR || in.op == FO_COUNT) fp.count_gword[fp.n_counts++] = in.c;
-      else if (in.op == FO_FIRSTROW) fp.first_gword = in.c;
-      else if (in.op == FO_SUM) {
-        fp.op_bits[fp.n_ops] = in.g;
-        fp.op_gword[fp.n_ops] = in.c;
-        fp.op_wide[fp.n_ops] = (in.a & 0x80) ? 1u : 0u;
-        ++fp.n_ops;
-      }
-    }
-    part_grid = (uint32_t)std::min<u64>((u64)ctx->sm_count, used);
+    lean.part_shift = a->packed.shift;
+    lean.part_dense = a->packed.dense;
+    r.fp = fold_plan(a);
+    r.part_grid = (uint32_t)std::min<u64>((u64)ctx->sm_count, used);
     a->info.partitions = (uint32_t)used;
-    a->info.packed_tuples = 1 + a->pk_dense;
-  } else if (partitioned) {
+    a->info.packed_tuples = 1 + a->packed.dense;
+  } else if (partition) {
     const u64 table_bytes = a->gcap * (8ull + 8ull * a->n_gwords);
     uint32_t cap_log2 = 0;
     while ((1ull << cap_log2) < a->gcap) ++cap_log2;
@@ -4160,68 +4172,26 @@ static int32_t agg_launch(llkv_gpu_agg* a, const llkv_gpu_program* prog, int app
     while (bits < 8 && (table_bytes >> bits) > (slice_mb << 20)) ++bits;
     if (bits + 3 > cap_log2) bits = cap_log2 > 3 ? cap_log2 - 3 : 1;
     const u64 P = 1ull << bits;
-    u64 batch_rows = 1ull << 28;
-    if (const char* e = getenv("LLKV_GPU_PART_BATCH_ROWS")) batch_rows = std::max<u64>(p.tile_rows, strtoull(e, nullptr, 10));  // tests: several launches on small tables
-    const u64 dense_max_rows = max_rows_per_launch;
-    u64 part_cap = 0;
-    for (;;) {  // the tuple buffers of one launch; when HBM is short the launches get smaller instead
-      max_rows_per_launch = std::max<u64>(p.tile_rows, std::min<u64>(dense_max_rows, batch_rows) / p.tile_rows * p.tile_rows);
-      const u64 launch_rows = std::min<u64>(row_end - row_begin + p.tile_rows, max_rows_per_launch);
-      part_cap = (launch_rows / P + launch_rows / (4 * P) + 1024 + 15) / 16 * 16;
-      const size_t elems = (size_t)(P * lean.s.n_fields * part_cap);
-      if (a->part_out_elems >= elems) break;
-      if (a->part_out) CUDA_TRY(cudaFree(a->part_out));
-      a->part_out = nullptr;
-      a->part_out_elems = 0;
-      if (cudaMalloc((void**)&a->part_out, elems * 8) == cudaSuccess) {
-        a->part_out_elems = elems;
-        break;
-      }
-      cudaGetLastError();
-      a->part_out = nullptr;
-      if (batch_rows <= (1ull << 22)) return set_error(LLKV_ERR_IO, "out of device memory for the tuple partitions of a GROUP BY (%zu bytes)", elems * 8);
-      batch_rows >>= 1;
-    }
-    if (!a->part_cursor) CUDA_TRY(cudaMalloc((void**)&a->part_cursor, kMaxPackedPartitions * 4));
-    lean.part_out = a->part_out;
-    lean.part_cursor = a->part_cursor;
-    lean.part_cap = part_cap;
+    if ((rc = agg_part_buffers(a, 1ull << 28, false, P, P * lean.s.n_fields, row_end - row_begin, r.max_rows))) return rc;
     lean.part_bits = bits;
     lean.part_shift = cap_log2 - bits;
-    memset(&pp, 0, sizeof(pp));
-    pp.tuples = a->part_out;
-    pp.cursor = a->part_cursor;
-    pp.part_cap = part_cap;
-    pp.gkeys = a->gkeys;
-    pp.gwords = a->gwords;
-    pp.gcap = a->gcap;
-    pp.flags = a->d_flags;
-    pp.n_parts = (uint32_t)P;
-    pp.n_fields = lean.s.n_fields;
-    pp.n_keys = lean.s.n_keys;
-    pp.n_gwords = lean.s.n_gwords;
-    pp.chunk = 2048;
-    pp.chunks_per_part = (uint32_t)((part_cap + pp.chunk - 1) / pp.chunk);
-    for (uint32_t i = 0; i < lean.s.n_code; ++i) {  // operand fields follow the order of the aggregates (lean_field_index)
-      const FInstr& in = lean.s.code[i];
-      if (in.op < FO_COUNT_STAR || in.op > FO_FIRSTNAN) continue;
-      PartOp& o = lean_takes_operand(in.op) ? pp.vops[pp.n_vops++] : pp.nops[pp.n_nops++];
-      o.op = in.op;
-      o.flags = in.a;
-      o.gword = in.c;
-    }
-    part_grid = (uint32_t)ctx->sm_count;  // launch_partition_apply multiplies by the kernel's resident CTAs per SM
+    r.pp = part_plan(a, (uint32_t)P);
+    r.part_grid = (uint32_t)ctx->sm_count;  // launch_partition_apply multiplies by the kernel's resident CTAs per SM
     a->info.partitions = (uint32_t)P;
-    a->info.packed_tuples = 0;
-  } else {
-    a->info.partitions = 0;
-    a->info.packed_tuples = 0;
   }
-  // Zone-map pruning (lean path): every FO_LEAF of the program is a conjunct (`selected &= lo <= v <= hi`), so a tile none
-  // of whose zones can satisfy some leaf holds no selected row.  The surviving tiles are listed on the host from the
-  // columns' zone maps and the launch walks the list instead of the dense tile range.
+  return LLKV_OK;
+}
+
+// Zone-map pruning (lean path): every FO_LEAF of the program is a conjunct (`selected &= lo <= v <= hi`), so a tile none
+// of whose zones can satisfy some leaf holds no selected row.  The surviving tiles are listed on the host from the
+// columns' zone maps and the launch walks the list instead of the dense tile range.  *use_tile_list: the run walks it.
+static int32_t agg_tile_list(llkv_gpu_agg* a, uint64_t sig, const std::vector<llkv_gpu_column*>& handles, uint64_t table_rows,
+                             uint64_t row_begin, uint64_t row_end, bool* use_tile_list) {
+  llkv_gpu_ctx* ctx = a->ctx;
+  const Plan& p = a->cr.plan;
+  const LeanPlan& lean = a->lean;
   a->info.tiles_pruned = 0;
-  bool use_tile_list = false;
+  bool use = false;
   if (a->cr.fast && ctx->prune_mode && row_end > row_begin) {
     struct PruneLeaf { llkv_gpu_column* col; i64 lo, hi; bool uns; };
     std::vector<PruneLeaf> leaves;
@@ -4247,7 +4217,7 @@ static int32_t agg_launch(llkv_gpu_agg* a, const llkv_gpu_program* prog, int app
       wanted = settled;
     }
     if (wanted && a->tile_list_key == key) {
-      use_tile_list = a->tile_list_use;
+      use = a->tile_list_use;
     } else if (wanted) {
       const u64 T = p.tile_rows;
       const u64 n_zones = (table_rows + kZoneRows - 1) / kZoneRows;
@@ -4255,7 +4225,8 @@ static int32_t agg_launch(llkv_gpu_agg* a, const llkv_gpu_program* prog, int app
       bool any_map = false;
       for (PruneLeaf& L : leaves) {
         bool ok = false;
-        if ((rc = ensure_zones(L.col, &ok))) return rc;
+        int32_t rc = ensure_zones(L.col, &ok);
+        if (rc) return rc;
         if (!ok || L.col->h_zones.size() != 2 * n_zones) continue;
         any_map = true;
         const u64* z = L.col->h_zones.data();
@@ -4290,26 +4261,36 @@ static int32_t agg_launch(llkv_gpu_agg* a, const llkv_gpu_program* prog, int app
         CUDA_TRY(cudaMemcpyAsync(a->d_tile_list, a->h_tile_list.data(), kept * 4, cudaMemcpyHostToDevice, ctx->stream));
         CUDA_TRY(cudaStreamSynchronize(ctx->stream));  // (h_tile_list is pageable; once per list)
       }
-      use_tile_list = a->tile_list_use;
+      use = a->tile_list_use;
     }
-    if (use_tile_list) a->info.tiles_pruned = (uint32_t)(a->tile_list_total - a->h_tile_list.size());
+    if (use) a->info.tiles_pruned = (uint32_t)(a->tile_list_total - a->h_tile_list.size());
   }
+  *use_tile_list = use;
+  return LLKV_OK;
+}
+
+// The launches of a run: dense row ranges, or runs of the tile list (bounded in tiles, and in the rows they span:
+// launch-relative row indices are 32-bit).  A partitioned scan launch is followed by the second pass of its form.
+static int32_t agg_run_launches(llkv_gpu_agg* a, uint64_t row_begin, uint64_t row_end, RunLaunches& r, uint32_t* launches_out) {
+  llkv_gpu_ctx* ctx = a->ctx;
+  const Plan& p = a->cr.plan;
+  LeanPlan& lean = a->lean;
+  const bool partitioned = a->cr.fast && lean.s.partition != 0;
+  const bool packed = a->cr.fast && lean.s.partition == 2;
   a->pending.timed = ctx->timing;
   if (ctx->timing) CUDA_TRY(cudaEventRecord(ctx->ev0, ctx->stream));
   uint32_t launches = 0;
   a->info.used_jit_kernel = 0;
   lean.tile_list = nullptr;
-  lean.s.use_tile_list = use_tile_list ? 1u : 0u;
-  // launches: dense row ranges, or runs of the tile list (bounded in tiles, and in the rows they span: launch-relative
-  // row indices are 32-bit)
-  const u64 list_n = use_tile_list ? a->h_tile_list.size() : 0;
-  const u64 tiles_per_launch = std::max<u64>(1, max_rows_per_launch / p.tile_rows);
+  lean.s.use_tile_list = r.use_tile_list ? 1u : 0u;
+  const u64 list_n = r.use_tile_list ? a->h_tile_list.size() : 0;
+  const u64 tiles_per_launch = std::max<u64>(1, r.max_rows / p.tile_rows);
   u64 list_pos = 0;
-  for (u64 rb = row_begin; use_tile_list || rb < row_end || (rb == row_begin && launches == 0); rb += max_rows_per_launch) {
-    u64 re = std::min<u64>(row_end, rb + max_rows_per_launch);
+  for (u64 rb = row_begin; r.use_tile_list || rb < row_end || (rb == row_begin && launches == 0); rb += r.max_rows) {
+    u64 re = std::min<u64>(row_end, rb + r.max_rows);
     u64 first_tile = rb / p.tile_rows;
     u64 n_tiles = re > rb ? (re + p.tile_rows - 1) / p.tile_rows - first_tile : 0;
-    if (use_tile_list) {
+    if (r.use_tile_list) {
       if (list_pos >= list_n) break;
       first_tile = a->h_tile_list[list_pos];
       n_tiles = 1;
@@ -4323,7 +4304,7 @@ static int32_t agg_launch(llkv_gpu_agg* a, const llkv_gpu_program* prog, int app
       list_pos += n_tiles;
     }
     if (n_tiles == 0) break;
-    const u64 grid = std::min<u64>(g.grid, n_tiles);
+    const u64 grid = std::min<u64>(r.g.grid, n_tiles);
     if (!launches) a->info.grid = (uint32_t)grid;
     if (a->cr.fast) {
       lean.row_begin = rb;
@@ -4332,14 +4313,14 @@ static int32_t agg_launch(llkv_gpu_agg* a, const llkv_gpu_program* prog, int app
       lean.n_tiles = n_tiles;
       bool jitted = false;
       if (partitioned) CUDA_TRY(cudaMemsetAsync(a->part_cursor, 0, kMaxPackedPartitions * 4, ctx->stream));
-      if (use_jit) CUDA_TRY(jit_launch(ctx->device, lean, (int)lean_ctas, (uint32_t)grid, ctx->stream, &jitted, nullptr));
+      if (r.use_jit) CUDA_TRY(jit_launch(ctx->device, lean, (int)r.lean_ctas, (uint32_t)grid, ctx->stream, &jitted, nullptr));
       if (partitioned) {
         if (!jitted) return set_error(LLKV_ERR_INTERNAL, "the partitioned scan needs its specialised kernel");
         if (packed) {
-          fp.row_base = lean.row_origin + first_tile * (u64)p.tile_rows;  // launch-relative row 0
-          CUDA_TRY(launch_partition_fold(fp, part_grid, ctx->stream));
+          r.fp.row_base = lean.row_origin + first_tile * (u64)p.tile_rows;  // launch-relative row 0
+          CUDA_TRY(launch_partition_fold(r.fp, r.part_grid, ctx->stream));
         } else {
-          CUDA_TRY(launch_partition_apply(pp, part_grid, ctx->stream));
+          CUDA_TRY(launch_partition_apply(r.pp, r.part_grid, ctx->stream));
         }
         ++launches;
       }
@@ -4354,12 +4335,59 @@ static int32_t agg_launch(llkv_gpu_agg* a, const llkv_gpu_program* prog, int app
       if (launches) CUDA_TRY(cudaStreamSynchronize(ctx->stream));  // h_plan is reused
       memcpy(a->h_plan, &lp, sizeof(Plan));
       CUDA_TRY(cudaMemcpyAsync(a->d_plan, a->h_plan, sizeof(Plan), cudaMemcpyHostToDevice, ctx->stream));
-      CUDA_TRY(launch_scan(a->d_plan, a->cr.wide, (int)g.R, (uint32_t)grid, g.block, g.smem, ctx->stream));
+      CUDA_TRY(launch_scan(a->d_plan, a->cr.wide, (int)r.g.R, (uint32_t)grid, r.g.block, r.g.smem, ctx->stream));
     }
     ++launches;
-    if (use_tile_list ? list_pos >= list_n : re >= row_end) break;
+    if (r.use_tile_list ? list_pos >= list_n : re >= row_end) break;
   }
   if (ctx->timing) CUDA_TRY(cudaEventRecord(ctx->ev1, ctx->stream));
+  *launches_out = launches;
+  return LLKV_OK;
+}
+
+static int32_t agg_launch(llkv_gpu_agg* a, const llkv_gpu_program* prog, int apply_mvcc, uint64_t row_begin, uint64_t row_end,
+                          bool force_wide) {
+  llkv_gpu_ctx* ctx = a->ctx;
+  CompileRequest req;
+  std::vector<llkv_gpu_column*> handles;
+  uint64_t table_rows = 0;
+  int32_t rc = build_request(ctx, a->table_id, prog, apply_mvcc, req, handles, &table_rows);
+  if (rc) return rc;
+  if (row_end > table_rows) return set_error(LLKV_ERR_INVALID_ARGUMENT, "row_end %llu beyond the table's %llu rows", (unsigned long long)row_end, (unsigned long long)table_rows);
+  // Multi-GPU GROUP BY: the packed key layout (bits, minimum, string length per key) comes from column statistics, and
+  // partial tables can only be merged key by key if every rank packs alike.  The ranks agree on the statistics of the
+  // key columns (min of minima, max of maxima / string lengths) with one small all-reduce before compiling.
+  if (ctx->nccl_comm && ctx->n_ranks > 1 && !a->keys.empty()) {
+    bool changed = false;
+    if ((rc = agree_dictionaries(ctx, a, handles, &changed))) return rc;
+    if (changed) {  // columns were re-coded: their descriptions again
+      req = CompileRequest();
+      handles.clear();
+      if ((rc = build_request(ctx, a->table_id, prog, apply_mvcc, req, handles, &table_rows))) return rc;
+    }
+    if ((rc = agree_key_stats(ctx, a, req))) return rc;
+  }
+  const unsigned char* exists_bits = nullptr;
+  if ((rc = table_exists_bits(ctx, a->table_id, handles, table_rows, &exists_bits))) return rc;
+  const uint64_t sig = request_signature(ctx, req, prog, force_wide, exists_bits);
+  RunLaunches r;
+  if ((rc = agg_compile(a, req, sig, force_wide, row_begin, row_end, r.g))) return rc;
+  a->cr.plan.exists_bits = exists_bits;
+  if (a->cr.fast && (rc = agg_choose_form(a, row_begin, row_end, r))) return rc;
+  if ((rc = agg_bind_state(a, handles))) return rc;
+  const bool need_backup = a->cr.can_narrow_fail || a->cr.plan.n_keys != 0;
+  if (need_backup && (rc = agg_backup(a))) return rc;
+  a->pending.has_backup = need_backup;
+  // thread-private partial sums stay exact while a thread folds a bounded number of rows per launch: split very long scans
+  // (general interpreter: < 2^15 rows per thread; lean kernel: 2^kLeanRowsPerThreadLog2 rows per consumer thread, and
+  // launch-relative row indices must fit 32 bits)
+  const uint32_t T = a->cr.plan.tile_rows;
+  r.max_rows = (u64)r.g.grid * r.g.block * 32000ull;
+  if (a->cr.fast) r.max_rows = std::min<u64>(r.max_rows, 0xf0000000ull) / T * T;
+  if ((rc = agg_partitions(a, req, row_begin, row_end, r))) return rc;
+  if ((rc = agg_tile_list(a, sig, handles, table_rows, row_begin, row_end, &r.use_tile_list))) return rc;
+  uint32_t launches = 0;
+  if ((rc = agg_run_launches(a, row_begin, row_end, r, &launches))) return rc;
   if (!a->skip_scan_copy && (rc = agg_queue_result_copy(a))) return rc;
   a->info.rows = row_end - row_begin;
   a->info.kernel_launches = launches;
@@ -4367,11 +4395,11 @@ static int32_t agg_launch(llkv_gpu_agg* a, const llkv_gpu_program* prog, int app
   a->info.used_fast_kernel = a->cr.fast ? 1 : 0;
   a->info.algorithmic_bytes_per_row = a->cr.algorithmic_bytes_per_row;
   a->info.physical_bytes_per_row = a->cr.physical_bytes_per_row;
-  a->info.block = g.block;
-  a->info.rows_per_tile = p.tile_rows;
-  a->info.stages = p.stages;
-  a->info.smem_bytes = g.smem;
-  a->info.fast_groups = p.fast_groups;
+  a->info.block = r.g.block;
+  a->info.rows_per_tile = T;
+  a->info.stages = a->cr.plan.stages;
+  a->info.smem_bytes = r.g.smem;
+  a->info.fast_groups = a->cr.plan.fast_groups;
   return LLKV_OK;
 }
 
@@ -4864,7 +4892,7 @@ static int32_t agg_collect(llkv_gpu_agg* a, std::vector<u64>& hk, std::vector<u6
   std::sort(groups.begin(), groups.end(), [](const GroupRef& x, const GroupRef& y) { return x.first_row < y.first_row; });
   if (a->hint && a->hint <= 128 && groups.size() > a->hint && groups.size() > a->observed_groups) {
     a->observed_groups = groups.size();  // the caller's hint was low: later runs of this aggregate get more CTA-local slots
-    a->lean_have[0] = a->lean_have[1] = a->lean_have[2] = a->lean_have[3] = false;
+    a->forget_forms();
     ++a->plan_epoch;
   }
   return LLKV_OK;
@@ -5249,7 +5277,7 @@ static bool merge_is_p2p(const llkv_gpu_agg* a) {
   if (!a->frozen || !ctx->nccl_comm || ctx->n_ranks < 2 || !ctx->p2p_merge) return false;
   if (a->cr.plan.n_keys == 0) return !a->cr.can_narrow_fail && a->n_gwords < 127;
   if (!a->hint || a->p2p_group_disabled) return false;
-  const u64 cap0 = next_pow2(std::max<u64>(32, a->hint * 2)) * 4;
+  const u64 cap0 = group_table_cap(a->hint) * 4;
   return 2 + cap0 + (cap0 + 2) * (a->n_gwords + 1) <= kGroupSlotWords;
 }
 
@@ -5299,7 +5327,7 @@ static int32_t agg_merge_impl(llkv_gpu_agg* a) {
   // peer-mailbox exchange, one kernel queued behind the scan, no collective, no host synchronisation.  The condition only
   // uses the hint and the accumulator layout, which every rank shares.
   if (a->frozen && a->cr.plan.n_keys != 0 && ctx->nccl_comm && N > 1 && ctx->p2p_merge && a->hint && !a->p2p_group_disabled) {
-    const u64 cap0 = next_pow2(std::max<u64>(32, a->hint * 2)) * 4;
+    const u64 cap0 = group_table_cap(a->hint) * 4;
     if (2 + cap0 + (cap0 + 2) * (a->n_gwords + 1) <= kGroupSlotWords) {
       if (!a->pending.active) {
         a->pending.active = true;

@@ -18,7 +18,7 @@ namespace llkv {
 
 constexpr int kMaxCols = 24;
 constexpr int kMaxInstr = 320;
-constexpr int kMaxFastInstr = 96;      // lean-kernel program (fast_kernel.cu)
+constexpr int kMaxFastInstr = 96;      // lean-kernel program (lean_kernel.cuh)
 constexpr int kMaxLits = 96;
 constexpr int kMaxNoncommitted = 32;
 constexpr int kMaxKeys = 8;
@@ -258,12 +258,11 @@ struct Plan {
   // ---- lean-kernel program (valid when n_finstr != 0)
   uint32_t n_finstr;
   uint32_t fast_tmps;             // tile-sized temporaries the lean program uses (<= kFastTmps)
-  uint32_t smem_tmp_off;          // their shared-memory offset (fast kernel)
   FInstr fcode[kMaxFastInstr];
   uint8_t key_col[kMaxKeys];      // plan column index of each GROUP BY key
   uint8_t key_load[kMaxKeys];     // its LoadKind
   // shared-memory layout (byte offsets from the dynamic smem base; all 128-byte aligned)
-  uint32_t smem_plan_off, smem_bar_off, smem_stage_off, smem_acc_off, smem_spill_off, smem_tbl_off, smem_total;
+  uint32_t smem_bar_off, smem_stage_off, smem_acc_off, smem_spill_off, smem_tbl_off, smem_total;
   // ---- global state
   unsigned long long* gkeys;      // [gcap] open addressing, kEmptyKey = free; group rows gcap (key == kEmptyKey) and gcap+1 (NULL key)
   unsigned long long* gwords;     // [(gcap+2) * n_gwords]

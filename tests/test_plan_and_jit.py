@@ -175,6 +175,18 @@ def test_partitioned_scan_compiles_for_sm_100a(tmp_path):
     assert int(usage.split("STACK:")[1].split()[0]) == 0
 
 
+def test_listing_partitions_only_where_the_runtime_does():
+    """The listing asks the runtime's form policy: a GROUP BY with a cardinality hint of 128 or less (or none) keeps its
+    CTA-local group slots and runs per row in every partitioning mode, so its listing shows no partitioned form."""
+    t = tpch.highcard_table(50_000, 20_000, seed=4)
+    for hint in (0, 1, 100, 128):
+        for kw in (dict(partition=True), dict(packed=True)):
+            text = gpu.debug_plan(t, None, tpch.highcard_aggregates(), group_by=(tpch.K_FIELD,), cardinality_hint=hint, **kw)
+            assert text.startswith("lean plan") and "partitioned" not in text, (hint, kw, text)
+    text = gpu.debug_plan(t, None, tpch.highcard_aggregates(), group_by=(tpch.K_FIELD,), cardinality_hint=129, partition=True)
+    assert "partitioned: 3 fields per tuple" in text, text
+
+
 def test_pinned_geometry_that_does_not_fit_keeps_the_group_slots(lineitem):
     """llkv_gpu_ctx_set_tuning may pin a geometry that does not fit in shared memory.  The fallback gives up consumer
     threads (whole warps) before CTA-local group slots: Q1's four groups keep their four slots."""
