@@ -400,9 +400,13 @@ int32_t llkv_gpu_column_reserve(llkv_gpu_column* col, uint64_t n_rows);
 /* Appends one chunk.  `values` is the Arrow values buffer (pager blob + 24, serialization.rs:41-53).
  * `validity` is an optional Arrow validity bitmap (LSB first) for the chunk; NULL = all valid (the
  * reference's chunk format stores no nulls, serialization.rs:265-269).  `row_ids` is the chunk's
- * row-id shadow column or NULL for the dense run starting at `row_id_base`.  Row ids must continue the
- * column densely (SURVEY.md §7 hard part (a)); anything else is LLKV_ERR_INVALID_ARGUMENT for now.
- * For LLKV_PT_UTF8 `values` is the i32 offsets buffer (n_rows+1) and `aux` the data bytes.
+ * row-id shadow column or NULL for the dense run starting at `row_id_base`.  Row ids that do not continue the column
+ * densely (rows appended after deletes, updates, columns that skip the rows where they are NULL) make the column
+ * row-id sparse: a row lands at position row id - the column's first row id (name the table's first row id in
+ * `row_id_base` with a first chunk of scattered ids), its validity bit is set, a row the chunk marks NULL is not written,
+ * and a row id written again takes the later chunk's value (last writer wins).  Row ids within one chunk must be distinct.
+ * For LLKV_PT_UTF8 `values` is the i32 offsets buffer (n_rows+1) and `aux` the data bytes, for dense and sparse chunks
+ * alike (see "Utf8 columns" below).
  * `values` may also point into device memory of the context's GPU (fixed-width types): the chunk is then copied device to
  * device in stream order, and the page-locked lifetime rule above applies to it. */
 int32_t llkv_gpu_column_append_chunk(llkv_gpu_column* col, uint64_t chunk_pk, const void* values, uint64_t n_rows,
@@ -435,6 +439,12 @@ int32_t llkv_gpu_column_gather(llkv_gpu_column* col, const uint64_t* row_ids, ui
  * expressions over a dictionary-coded column are LLKV_ERR_INVALID_ARGUMENT.  Across GPUs the ranks agree on one dictionary
  * per Utf8 key column before a grouped plan is compiled (an all-gather of their entries; a rank whose shard holds short
  * strings only switches to dictionary form with the others), so codes mean the same string on every rank.
+ * Row-id-sparse chunks (llkv_gpu_column_append_chunk) take the same forms: short strings are packed on the device as they
+ * are scattered to their positions; a chunk with a longer string re-codes the column (only the strings of rows that exist
+ * are interned: a gap or a deleted row adds no entry) and later chunks are interned on the host and scattered as codes.
+ * A string replaced by a later write, or whose rows were deleted, stays in the dictionary until llkv_gpu_column_clear.
+ * At seal the statistics of a sparse short-string column (longest and shortest string, non-ASCII bytes) are recomputed
+ * over the rows that exist, so a column whose present strings are all one byte long is kept at one byte per row.
  * llkv_gpu_column_dict_entry: the bytes stay valid until the next append to / clear of the column. */
 int32_t llkv_gpu_column_dict_size(llkv_gpu_column* col, uint64_t* out_entries);
 int32_t llkv_gpu_column_dict_entry(llkv_gpu_column* col, uint64_t code, const uint8_t** out_bytes, uint64_t* out_len);

@@ -276,6 +276,74 @@ __global__ void scatter_rows_kernel(T* __restrict__ dst, unsigned int* __restric
     atomicOr(&valid[pos >> 5], 1u << (pos & 31));
   }
 }
+// Block-wide max / min string length and bad-string bits (1: longer than 7 bytes, 2: a byte >= 0x80) folded into *st with
+// one atomic per field.  Every thread of the block calls it; blockDim.x is a multiple of 32, at most 1024.
+__device__ __forceinline__ void block_str_stats(unsigned int mx, unsigned int mn, unsigned int bad, DevStats* st) {
+  __shared__ unsigned int s_mx[32], s_mn[32], s_bad[32];
+  mx = __reduce_max_sync(0xffffffffu, mx);
+  mn = __reduce_min_sync(0xffffffffu, mn);
+  bad = __reduce_or_sync(0xffffffffu, bad);
+  const unsigned int w = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  if ((threadIdx.x & 31) == 0) {
+    s_mx[w] = mx;
+    s_mn[w] = mn;
+    s_bad[w] = bad;
+  }
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (unsigned int i = 1; i < nw; ++i) {
+      mx = s_mx[i] > mx ? s_mx[i] : mx;
+      mn = s_mn[i] < mn ? s_mn[i] : mn;
+      bad |= s_bad[i];
+    }
+    if (mx || mn != 0xffffffffu) {
+      atomicMax(&st->max_strlen, mx);
+      atomicMin(&st->min_strlen, mn);
+    }
+    if (bad) atomicOr(&st->bad_string, bad);
+  }
+}
+// Row-id-sparse appends of a packed Utf8 column: the rules of scatter_rows_kernel, with each string packed into its 8-byte
+// key on the way (as pack_utf8_kernel: `data` is the chunk's slice of the data buffer, offsets are relative to `first`).
+// Lengths and bytes of the rows written feed the statistics.
+__global__ void scatter_utf8_kernel(u64* __restrict__ dst, unsigned int* __restrict__ valid, const int* __restrict__ off,
+                                    const unsigned char* __restrict__ data, int first, const u64* __restrict__ ids,
+                                    const unsigned char* __restrict__ src_valid, u64 n, u64 origin, DevStats* st) {
+  unsigned int mx = 0, mn = 0xffffffffu, bad = 0;
+  for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
+    if (src_valid && !((src_valid[i >> 3] >> (i & 7)) & 1)) continue;
+    const int b = off[i] - first, e = off[i + 1] - first;
+    const unsigned int len = (unsigned int)(e - b);
+    u64 k = 0;
+    if (len > 7) bad |= 1;
+    else {
+      for (unsigned int j = 0; j < len; ++j) k |= (u64)data[b + j] << (56 - 8 * j);
+      k |= len;
+    }
+    const u64 pos = ids[i] - origin;
+    dst[pos] = k;
+    atomicOr(&valid[pos >> 5], 1u << (pos & 31));
+    if (k & 0x8080808080808000ull) bad |= 2;
+    mx = len > mx ? len : mx;
+    mn = len < mn ? len : mn;
+  }
+  block_str_stats(mx, mn, bad, st);
+}
+// Statistics of a packed Utf8 column over the positions whose validity bit is set (a sparse column at seal: gaps, deleted
+// rows and overwritten values must not count).  The length is the key's low byte, the bytes are the key's upper bytes.
+__global__ void str_stats_kernel(const u64* __restrict__ keys, const unsigned int* __restrict__ valid, u64 n, DevStats* st) {
+  unsigned int mx = 0, mn = 0xffffffffu, bad = 0;
+  for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
+    if (valid && !((valid[i >> 5] >> (i & 31)) & 1u)) continue;
+    const u64 k = keys[i];
+    const unsigned int len = (unsigned int)(k & 0xff);
+    if (len > 7) bad |= 1;
+    if (k & 0x8080808080808000ull) bad |= 2;
+    mx = len > mx ? len : mx;
+    mn = len < mn ? len : mn;
+  }
+  block_str_stats(mx, mn, bad, st);
+}
 // ColumnStore::delete_rows (store/core.rs:1392-1776): the rows leave the column; their positions stay as gaps
 __global__ void clear_rows_kernel(unsigned int* __restrict__ valid, const u64* __restrict__ ids, u64 n, u64 origin, u64 n_rows) {
   for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
@@ -1419,7 +1487,7 @@ static int32_t launch_stats(llkv_gpu_column* col, uint64_t first_row, uint64_t n
     case LLKV_PT_UINT32: stats_kernel<unsigned int, false><<<blocks, 256, 0, s>>>((const unsigned int*)base, n, col->dstats); break;
     case LLKV_PT_UINT64: stats_kernel<u64, false><<<blocks, 256, 0, s>>>((const u64*)base, n, col->dstats); break;
     case LLKV_PT_DECIMAL128: stats_dec_kernel<<<blocks, 256, 0, s>>>((const ulonglong2*)base, n, col->dstats); break;
-    default: return LLKV_OK;  // floats: no statistics needed; Utf8: gathered by the pack kernel
+    default: return LLKV_OK;  // floats: no statistics needed; Utf8: gathered by the pack kernel (str_stats_kernel at seal when sparse)
   }
   CUDA_TRY(cudaGetLastError());
   return LLKV_OK;
@@ -1554,11 +1622,44 @@ static UploadPool* upload_pool(llkv_gpu_ctx* c) {
   return c->pool.get();
 }
 
+// A Utf8 chunk (offsets n_rows + 1 in `off`, data bytes in `aux`) is checked on the host before anything is uploaded.
+static int32_t utf8_chunk_shape(const int32_t* off, uint64_t n_rows, const void* aux, SrcKind src_kind, int64_t* first, int64_t* data_bytes,
+                                bool* has_long) {
+  if (src_kind == SRC_DEVICE) return set_error(LLKV_ERR_INVALID_ARGUMENT, "Utf8 chunks must come from host memory (the offsets are validated on the host)");
+  *first = off[0];
+  *data_bytes = (int64_t)off[n_rows] - *first;
+  if (*first < 0 || *data_bytes < 0) return set_error(LLKV_ERR_INVALID_ARGUMENT, "Utf8 offsets are negative or not monotonic");
+  *has_long = false;
+  for (uint64_t i = 0; i < n_rows; ++i) {
+    if (off[i + 1] < off[i]) return set_error(LLKV_ERR_INVALID_ARGUMENT, "Utf8 offsets are not monotonic at row %llu", (unsigned long long)i);
+    *has_long = *has_long || off[i + 1] - off[i] > 7;
+  }
+  if (*data_bytes && !aux) return set_error(LLKV_ERR_INVALID_ARGUMENT, "Utf8 data buffer is NULL");
+  return LLKV_OK;
+}
+
+// Host side of an append to a dictionary-coded column: the chunk's valid strings are interned, codes[i] is row i's code
+// (0 under a NULL: the row's validity bit stays clear).
+static int32_t intern_chunk(StrDict& d, const int32_t* off, const char* data, const uint8_t* validity, uint64_t n_rows, std::vector<u64>& codes) {
+  codes.resize((size_t)n_rows);
+  for (uint64_t i = 0; i < n_rows; ++i) {
+    const bool valid = !validity || ((validity[i >> 3] >> (i & 7)) & 1);
+    codes[(size_t)i] = valid ? d.code_of(d.intern(data + off[i], (size_t)(off[i + 1] - off[i]))) : 0;
+  }
+  if (d.strings.size() > kMaxDictEntries) return set_error(LLKV_ERR_INVALID_ARGUMENT, "more than %zu distinct strings in a dictionary-coded column", kMaxDictEntries);
+  return LLKV_OK;
+}
+
+static int32_t widen_str8(llkv_gpu_column* col);
+static int32_t enter_dict_mode(llkv_gpu_column* col);
+
 // A chunk whose row ids do not continue the column densely (rows appended after deletes, updates of existing rows, columns
-// that skip rows because the value is NULL): positions are row id - origin, rows nobody wrote are invalid bits.
-static int32_t append_sparse(llkv_gpu_column* col, const void* values, uint64_t n_rows, const uint8_t* validity, const uint64_t* row_ids) {
+// that skip rows because the value is NULL): positions are row id - origin, rows nobody wrote are invalid bits.  Utf8 chunks
+// are packed into 8-byte keys by scatter_utf8_kernel, or interned on the host and scattered as codes once the column is
+// dictionary-coded.
+static int32_t append_sparse(llkv_gpu_column* col, const void* values, uint64_t n_rows, const uint8_t* validity, const uint64_t* row_ids,
+                             const void* aux) {
   llkv_gpu_ctx* c = col->ctx;
-  if (col->type == LLKV_PT_UTF8) return set_error(LLKV_ERR_INVALID_ARGUMENT, "Utf8 columns take dense row-id runs only");
   uint64_t lo = ~0ull, hi = 0;
   for (uint64_t i = 0; i < n_rows; ++i) {
     lo = std::min(lo, row_ids[i]);
@@ -1569,20 +1670,38 @@ static int32_t append_sparse(llkv_gpu_column* col, const void* values, uint64_t 
                      (unsigned long long)lo, (unsigned long long)col->row_id_origin);
   const uint64_t span = hi - col->row_id_origin + 1;
   if (span > (1ull << 40)) return set_error(LLKV_ERR_INVALID_ARGUMENT, "row ids span %llu positions: too sparse for a resident image", (unsigned long long)span);
+  const bool utf8 = col->type == LLKV_PT_UTF8;
+  const int32_t* off = (const int32_t*)values;
+  int64_t first = 0, data_bytes = 0;
+  bool has_long = false;
   int32_t rc;
+  if (utf8 && (rc = utf8_chunk_shape(off, n_rows, aux, source_kind(values), &first, &data_bytes, &has_long))) return rc;
   if ((rc = flush_upload(col)) || (rc = drain_jobs(col))) return rc;
   if (is_narrow_decimal(col) && (rc = widen_decimal(col, col->n_rows))) return rc;
+  if (col->load_kind == LK_STR8 && (rc = widen_str8(col))) return rc;  // sealed as one byte per string: back to packed keys
+  if (has_long && !col->dict && (rc = enter_dict_mode(col))) return rc;
+  std::vector<u64> codes;
+  if (utf8 && col->dict && (rc = intern_chunk(*col->dict, off, (const char*)aux, validity, n_rows, codes))) return rc;
+  const bool packed_utf8 = utf8 && !col->dict;
   col->sealed = false;
   const uint64_t new_rows = std::max<uint64_t>(col->n_rows, span);
   if ((rc = column_grow(col, new_rows))) return rc;
   if ((rc = ensure_validity(col))) return rc;  // rows so far are valid, everything behind them is not (yet)
   cudaStream_t s = c->copy_streams[(size_t)col->stream_index];
-  void* d_vals = nullptr;
+  void* d_vals = nullptr;  // values, codes, or a packed column's offsets
+  unsigned char* d_data = nullptr;
   u64* d_ids = nullptr;
   unsigned char* d_bits = nullptr;
-  CUDA_TRY(cudaMalloc(&d_vals, n_rows * col->elem_bytes));
+  const uint64_t val_bytes = packed_utf8 ? (n_rows + 1) * 4 : n_rows * col->elem_bytes;
+  CUDA_TRY(cudaMalloc(&d_vals, val_bytes));
   CUDA_TRY(cudaMalloc((void**)&d_ids, n_rows * 8));
-  if ((rc = upload(col, d_vals, values, n_rows * col->elem_bytes, source_kind(values)))) return rc;
+  if (utf8 && col->dict) rc = upload(col, d_vals, codes.data(), val_bytes, SRC_PAGEABLE);
+  else rc = upload(col, d_vals, values, val_bytes, source_kind(values));
+  if (rc) return rc;
+  if (packed_utf8 && data_bytes > 0) {  // the chunk's slice of the data buffer
+    CUDA_TRY(cudaMalloc((void**)&d_data, (size_t)data_bytes));
+    if ((rc = upload(col, d_data, (const char*)aux + first, (uint64_t)data_bytes, source_kind(aux)))) return rc;
+  }
   if ((rc = upload(col, d_ids, row_ids, n_rows * 8, source_kind(row_ids)))) return rc;
   if (validity) {
     CUDA_TRY(cudaMalloc((void**)&d_bits, (n_rows + 7) / 8));
@@ -1591,18 +1710,25 @@ static int32_t append_sparse(llkv_gpu_column* col, const void* values, uint64_t 
   if ((rc = flush_upload(col))) return rc;
   const unsigned blocks = (unsigned)std::min<uint64_t>((n_rows + 255) / 256, 1184);
   const u64 origin = col->row_id_origin;
-  switch (col->elem_bytes) {
-    case 1: scatter_rows_kernel<unsigned char><<<blocks, 256, 0, s>>>((unsigned char*)col->values, col->validity, (const unsigned char*)d_vals, d_ids, d_bits, n_rows, origin); break;
-    case 2: scatter_rows_kernel<unsigned short><<<blocks, 256, 0, s>>>((unsigned short*)col->values, col->validity, (const unsigned short*)d_vals, d_ids, d_bits, n_rows, origin); break;
-    case 4: scatter_rows_kernel<unsigned int><<<blocks, 256, 0, s>>>((unsigned int*)col->values, col->validity, (const unsigned int*)d_vals, d_ids, d_bits, n_rows, origin); break;
-    case 8: scatter_rows_kernel<u64><<<blocks, 256, 0, s>>>((u64*)col->values, col->validity, (const u64*)d_vals, d_ids, d_bits, n_rows, origin); break;
-    default: scatter_rows_kernel<ulonglong2><<<blocks, 256, 0, s>>>((ulonglong2*)col->values, col->validity, (const ulonglong2*)d_vals, d_ids, d_bits, n_rows, origin); break;
+  if (packed_utf8) {
+    scatter_utf8_kernel<<<blocks, 256, 0, s>>>((u64*)col->values, col->validity, (const int*)d_vals, d_data, (int)first, d_ids, d_bits, n_rows, origin,
+                                               col->dstats);
+  } else {
+    switch (col->elem_bytes) {
+      case 1: scatter_rows_kernel<unsigned char><<<blocks, 256, 0, s>>>((unsigned char*)col->values, col->validity, (const unsigned char*)d_vals, d_ids, d_bits, n_rows, origin); break;
+      case 2: scatter_rows_kernel<unsigned short><<<blocks, 256, 0, s>>>((unsigned short*)col->values, col->validity, (const unsigned short*)d_vals, d_ids, d_bits, n_rows, origin); break;
+      case 4: scatter_rows_kernel<unsigned int><<<blocks, 256, 0, s>>>((unsigned int*)col->values, col->validity, (const unsigned int*)d_vals, d_ids, d_bits, n_rows, origin); break;
+      case 8: scatter_rows_kernel<u64><<<blocks, 256, 0, s>>>((u64*)col->values, col->validity, (const u64*)d_vals, d_ids, d_bits, n_rows, origin); break;
+      default: scatter_rows_kernel<ulonglong2><<<blocks, 256, 0, s>>>((ulonglong2*)col->values, col->validity, (const ulonglong2*)d_vals, d_ids, d_bits, n_rows, origin); break;
+    }
   }
   CUDA_TRY(cudaGetLastError());
   CUDA_TRY(cudaFreeAsync(d_vals, s));
   CUDA_TRY(cudaFreeAsync(d_ids, s));
+  if (d_data) CUDA_TRY(cudaFreeAsync(d_data, s));
   if (d_bits) CUDA_TRY(cudaFreeAsync(d_bits, s));
   CUDA_TRY(cudaStreamSynchronize(s));  // (the sources were pageable staging copies or page-locked: either way they are free now)
+  if (utf8) col->hstats.data_bytes += (u64)data_bytes;
   col->n_rows = new_rows;
   col->sparse = true;
   ++col->version;
@@ -1627,7 +1753,8 @@ static int32_t widen_str8(llkv_gpu_column* col) {
 }
 
 // A Utf8 column meets its first string longer than 7 bytes: the rows it already holds (packed keys, which carry their bytes)
-// are read back once, interned, and rewritten as dictionary codes.
+// are read back once, interned, and rewritten as dictionary codes.  Only positions whose validity bit is set are interned:
+// a gap, a deleted row or a NULL holds no string (its code is 0 under a clear bit).
 static int32_t enter_dict_mode(llkv_gpu_column* col) {
   llkv_gpu_ctx* c = col->ctx;
   int32_t rc = flush_upload(col);
@@ -1640,8 +1767,18 @@ static int32_t enter_dict_mode(llkv_gpu_column* col) {
   if (col->n_rows) {
     std::vector<u64> keys((size_t)col->n_rows);
     CUDA_TRY(cudaMemcpy(keys.data(), col->values, col->n_rows * 8, cudaMemcpyDeviceToHost));
+    std::vector<unsigned int> bits;
+    if (col->validity) {
+      bits.resize((size_t)((col->n_rows + 31) / 32));
+      CUDA_TRY(cudaMemcpy(bits.data(), col->validity, bits.size() * 4, cudaMemcpyDeviceToHost));
+    }
     std::unordered_map<u64, uint32_t> seen;
-    for (u64& k : keys) {
+    for (size_t i = 0; i < keys.size(); ++i) {
+      u64& k = keys[i];
+      if (!bits.empty() && !((bits[i >> 5] >> (i & 31)) & 1u)) {
+        k = 0;
+        continue;
+      }
       auto it = seen.find(k);
       if (it == seen.end()) {
         char b[8];
@@ -1706,7 +1843,7 @@ static int32_t append_chunk_impl(llkv_gpu_column* col, const void* values, uint6
       return set_error(LLKV_ERR_INVALID_ARGUMENT, "chunk row ids start at %llu but the column continues at %llu: pass the row ids of a chunk that does not continue the column",
                        (unsigned long long)first_id, (unsigned long long)(col->row_id_origin + col->n_rows));
     if (n_rows == 0) return LLKV_OK;
-    return append_sparse(col, values, n_rows, validity, row_ids);
+    return append_sparse(col, values, n_rows, validity, row_ids, aux);
   }
   if (n_rows == 0) return LLKV_OK;
   col->sealed = false;
@@ -1745,30 +1882,18 @@ static int32_t append_chunk_impl(llkv_gpu_column* col, const void* values, uint6
   }
   if ((rc = column_grow(col, col->n_rows + n_rows))) return rc;
   cudaStream_t s = c->copy_streams[(size_t)col->stream_index];
-  if (col->type == LLKV_PT_UTF8 && src_kind == SRC_DEVICE) return set_error(LLKV_ERR_INVALID_ARGUMENT, "Utf8 chunks must come from host memory (the offsets are validated on the host)");
   if (col->type == LLKV_PT_UTF8) {
     // the chunk's slice of the data buffer is uploaded and the offsets are rebased on the device (a column appended in many
     // chunks from one data buffer uploads every byte once)
     const int32_t* off = (const int32_t*)values;
-    const int64_t first = off[0], data_bytes = (int64_t)off[n_rows] - first;
-    if (first < 0 || data_bytes < 0) return set_error(LLKV_ERR_INVALID_ARGUMENT, "Utf8 offsets are negative or not monotonic");
-    bool has_long = false;
-    for (uint64_t i = 0; i < n_rows; ++i) {
-      if (off[i + 1] < off[i]) return set_error(LLKV_ERR_INVALID_ARGUMENT, "Utf8 offsets are not monotonic at row %llu", (unsigned long long)i);
-      has_long = has_long || off[i + 1] - off[i] > 7;
-    }
-    if (data_bytes && !aux) return set_error(LLKV_ERR_INVALID_ARGUMENT, "Utf8 data buffer is NULL");
+    int64_t first, data_bytes;
+    bool has_long;
+    if ((rc = utf8_chunk_shape(off, n_rows, aux, src_kind, &first, &data_bytes, &has_long))) return rc;
     if (has_long && !col->dict && (rc = enter_dict_mode(col))) return rc;
     if (col->dict) {
       // the host interns every string; 8 bytes of code per row cross the link, the bytes of the strings never do
-      StrDict& d = *col->dict;
-      std::vector<u64> codes((size_t)n_rows);
-      const char* data = (const char*)aux;
-      for (uint64_t i = 0; i < n_rows; ++i) {
-        const bool valid = !validity || ((validity[i >> 3] >> (i & 7)) & 1);
-        codes[(size_t)i] = valid ? d.code_of(d.intern(data + off[i], (size_t)(off[i + 1] - off[i]))) : 0;
-      }
-      if (d.strings.size() > kMaxDictEntries) return set_error(LLKV_ERR_INVALID_ARGUMENT, "more than %zu distinct strings in a dictionary-coded column", kMaxDictEntries);
+      std::vector<u64> codes;
+      if ((rc = intern_chunk(*col->dict, off, (const char*)aux, validity, n_rows, codes))) return rc;
       if ((rc = upload(col, (u64*)col->values + col->n_rows, codes.data(), n_rows * 8, SRC_PAGEABLE))) return rc;
       if ((rc = flush_upload(col))) return rc;
       CUDA_TRY(cudaStreamSynchronize(s));  // `codes` goes away with this scope
@@ -1928,8 +2053,15 @@ extern "C" int32_t llkv_gpu_column_seal(llkv_gpu_column* col) {
     memset(&init, 0, sizeof(init));
     init.min_enc = ~0ull;
     init.min_strlen = 0xffffffffu;
-    CUDA_TRY(cudaMemcpy(col->dstats, &init, sizeof(init), cudaMemcpyHostToDevice));
+    cudaStream_t ss = c->copy_streams[(size_t)col->stream_index];
+    CUDA_TRY(cudaMemcpyAsync(col->dstats, &init, sizeof(init), cudaMemcpyHostToDevice, ss));
     col->stats_rows = 0;
+    if (col->type == LLKV_PT_UTF8 && !col->dict && col->n_rows) {  // packed keys: lengths and bytes of the rows that exist
+      const unsigned blocks = (unsigned)std::min<uint64_t>((col->n_rows + 1023) / 1024, 1184);
+      str_stats_kernel<<<blocks, 256, 0, ss>>>((const u64*)col->values, col->validity, col->n_rows, col->dstats);
+      CUDA_TRY(cudaGetLastError());
+    }
+    CUDA_TRY(cudaStreamSynchronize(ss));
   }
   if (col->stats_rows < col->n_rows && col->load_kind != LK_STR8) {  // min / max / fits-i64 over the rows appended since the last seal
     int32_t rc = launch_stats(col, col->stats_rows, col->n_rows - col->stats_rows);
@@ -2649,7 +2781,8 @@ static uint64_t lfid_table(uint64_t lfid) { return (lfid >> 32) & 0xffffull; }  
 static uint64_t lfid_field(uint64_t lfid) { return lfid & 0xffffffffull; }
 
 // Row-id-sparse tables: every column covers positions [0, n) of the table's row-id range.  A column whose last rows are
-// absent (NULL by absence) is shorter than the others: it grows to the table's span, the new positions invalid.
+// absent (NULL by absence) is shorter than the others: it grows to the table's span, the new positions invalid (Utf8 columns
+// too, in whichever form they are resident: packed keys, one byte per row or dictionary codes).
 static int32_t equalise_sparse_columns(llkv_gpu_ctx* ctx, uint64_t table_id) {
   uint64_t longest = 0;
   bool differ = false, any = false;
@@ -2667,7 +2800,7 @@ static int32_t equalise_sparse_columns(llkv_gpu_ctx* ctx, uint64_t table_id) {
   if (!sparse_table) return LLKV_OK;  // dense tables keep the old rule: scans cover the rows every column has
   for (auto& kv : ctx->columns) {
     llkv_gpu_column* col = kv.second;
-    if (lfid_table(col->lfid) != (table_id & 0xffffull) || col->n_rows == longest || col->type == LLKV_PT_UTF8) continue;
+    if (lfid_table(col->lfid) != (table_id & 0xffffull) || col->n_rows == longest) continue;
     int32_t rc;
     if ((rc = column_flush(col))) return rc;
     if (is_narrow_decimal(col) && (rc = widen_decimal(col, col->n_rows))) return rc;

@@ -293,14 +293,18 @@ class DeviceColumn:
         _check(self.lib.llkv_gpu_column_append_chunk(self.handle, self.next_pk, C.c_void_p(ptr), n_rows, None, None, row_id_base, None))
         self.next_pk += 1
 
-    def append_rows(self, values: np.ndarray, row_ids: np.ndarray, first_row_id: int = 0, validity: Optional[np.ndarray] = None):
+    def append_rows(self, values: np.ndarray, row_ids: np.ndarray, first_row_id: int = 0, validity: Optional[np.ndarray] = None,
+                    aux: Optional[np.ndarray] = None):
         """One chunk with its row-id shadow column (ColumnStore::append with arbitrary row ids): rows land at position
-        row id - first_row_id; a row id that is already there is overwritten (last writer wins)."""
-        vals = np.ascontiguousarray(values)
+        row id - first_row_id; a row id that is already there is overwritten (last writer wins).  For a Utf8 column
+        `values` is the chunk's int32 offsets (one more than the row ids) and `aux` its data bytes."""
+        vals = np.ascontiguousarray(values, dtype=np.int32) if self.dtype.type == ffi.PT_UTF8 else np.ascontiguousarray(values)
         ids = np.ascontiguousarray(row_ids, dtype=np.uint64)
         vptr = C.c_void_p(validity.ctypes.data) if validity is not None else None
+        data = np.ascontiguousarray(aux, dtype=np.uint8) if aux is not None else None
+        aptr = C.c_void_p(data.ctypes.data) if data is not None and data.size else None
         _check(self.lib.llkv_gpu_column_append_chunk(self.handle, self.next_pk, C.c_void_p(vals.ctypes.data), ids.shape[0], vptr,
-                                                      C.c_void_p(ids.ctypes.data), first_row_id, None))
+                                                      C.c_void_p(ids.ctypes.data), first_row_id, aptr))
         self.next_pk += 1
 
     def delete_rows(self, row_ids):
