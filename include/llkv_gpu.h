@@ -601,7 +601,7 @@ int32_t llkv_gpu_debug_plan(const llkv_debug_column* cols, int32_t n_cols, const
                             int32_t deleted_by_col, uint64_t txn_id, uint64_t snapshot_id, const llkv_agg_spec* specs, int32_t n_aggs,
                             const llkv_scalar_node* nodes, int32_t n_nodes, const uint64_t* group_key_fields, int32_t n_keys,
                             int32_t expr_mode, uint64_t cardinality_hint, int32_t block_threads, int32_t rows_per_thread, int32_t stages,
-                            int32_t ctas_per_sm, int32_t jit /* bit 0: specialise with NVRTC, bit 1: as the partitioned GROUP BY scan, bit 2: as the scan that walks a tile list, bit 3: the partitioned scan with packed tuples */, const char* cubin_path, char* out_text, uint64_t out_cap);
+                            int32_t ctas_per_sm, int32_t jit /* bit 0: specialise with NVRTC, bit 1: as the partitioned GROUP BY scan, bit 2: as the scan that walks a tile list, bit 3: the partitioned scan with packed tuples, bit 4: the step form of a run that continues the previous one without a reset */, const char* cubin_path, char* out_text, uint64_t out_cap);
 
 /* ---- multi-GPU: one context per rank, NCCL over NVLink (SURVEY.md §8e) ---- */
 #define LLKV_GPU_UNIQUE_ID_BYTES 128

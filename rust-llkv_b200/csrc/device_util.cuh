@@ -15,6 +15,11 @@ typedef unsigned long long u64;
 typedef __int128 i128;
 typedef unsigned __int128 u128;
 
+// the value an accumulator word of class `c` (WordClass) holds before any row is folded into it
+__device__ __forceinline__ u64 gword_initial(uint8_t c) {
+  return (c == WC_MIN || c == WC_MIN128 || c == WC_PAIR_LO_MIN) ? ~0ull : 0ull;
+}
+
 // ------------------------------------------------------------------ mbarrier + cp.async.bulk (TMA 1-D bulk copy)
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 

@@ -1345,6 +1345,33 @@ struct LeanTile {
   }
 };
 
+// The publishing epilogue (LeanPlan::publish): every CTA has folded into the table; the one that draws the last ticket
+// copies the status word and the table to page-locked host memory and re-arms the state for the next step, so a repeated
+// step is this one kernel.  `s_flag`: a shared word the fold no longer reads.  A global ticket and a plain shared store
+// (no shared atomics).
+__device__ __forceinline__ void lean_publish(const LeanPlan& p, const LeanShape& S, u64* s_flag) {
+  const uint32_t tid = threadIdx.x;
+  __threadfence();  // this thread's table updates and status bits, before its CTA's ticket
+  __syncthreads();
+  if (tid == 0) *s_flag = atomicAdd(p.ticket, 1u) == gridDim.x - 1 ? 1ull : 0ull;
+  __syncthreads();
+  if (!*s_flag) return;
+  __threadfence();
+  const uint32_t n_words = (uint32_t)(p.gcap + 2) * S.n_gwords, n_keys = S.n_keys ? (uint32_t)p.gcap : 0u;
+  u64* const out = p.publish;
+  if (tid == 0) out[0] = __ldcg(p.flags);
+  for (uint32_t i = tid; i < n_words; i += blockDim.x) out[1 + i] = __ldcg(&p.gwords[i]);
+  for (uint32_t i = tid; i < n_keys; i += blockDim.x) out[1 + n_words + i] = __ldcg(&p.gkeys[i]);
+  __threadfence_system();
+  __syncthreads();  // every read of the state is done before it is re-armed
+  for (uint32_t i = tid; i < n_words; i += blockDim.x) p.gwords[i] = gword_initial(p.gclass[i % S.n_gwords]);
+  for (uint32_t i = tid; i < n_keys; i += blockDim.x) p.gkeys[i] = kEmptyKey;
+  if (tid == 0) {
+    *p.flags = 0;
+    *p.ticket = 0;
+  }
+}
+
 template <int R, class Cfg>
 __device__ __forceinline__ void lean_body(const LeanPlan& p) {
   extern __shared__ __align__(128) unsigned char smem[];
@@ -1551,6 +1578,9 @@ __device__ __forceinline__ void lean_body(const LeanPlan& p) {
     }
   }
   if (errbits) atomicOr(p.flags, errbits);
+  if constexpr (!Cfg::kPartition) {
+    if (p.publish) lean_publish(p, S, gslot_s);
+  }
 }
 
 }  // namespace llkv

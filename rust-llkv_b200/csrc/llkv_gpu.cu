@@ -886,6 +886,7 @@ struct PendingRun {
   bool timed = false;
   bool is_merge = false;  // a grouped peer-mailbox merge is queued behind the run (agg_resolve settles both)
   bool timed_merge = false;
+  bool from_reset = false;  // the run started from the initial state: a rerun re-initialises instead of restoring a backup
 };
 
 // The forms a lean plan runs in: the interpreting build, the build specialised on the plan shape, and the two partitioned
@@ -964,6 +965,13 @@ struct llkv_gpu_agg {
   unsigned char* h_stage = nullptr;  // pinned landing buffer of finalize (small tables)
   size_t h_stage_bytes = 0;
   bool prefetched = false;  // h_stage holds the table as the last run left it (copy queued right behind the scan)
+  // One-kernel steps (step_publishes): `armed` = in stream order the status word, ticket and table hold their initial values,
+  // so a reset queues nothing.  `published` = the last run's scan copied its status word and table to h_pub (page-locked,
+  // mapped: [status][words][keys]) and re-armed the device state; h_pub is the result until something continues from it.
+  bool armed = false;
+  bool published = false;
+  u64* h_pub = nullptr;
+  u64* d_pub = nullptr;
   cudaEvent_t stage_ev = nullptr;  // recorded behind that copy
   Plan* d_plan = nullptr;
   Plan* h_plan = nullptr;  // pinned
@@ -979,6 +987,8 @@ struct llkv_gpu_agg {
   uint64_t graph_key = 0;
   PendingRun graph_pending;     // the pending-run bookkeeping of the captured step (without the program copy)
   bool graph_prefetched = false;
+  bool graph_from_armed = false;  // the captured step has no reset launches: it replays only onto an armed state
+  bool graph_published = false, graph_armed_after = false;
   uint32_t graph_launches = 0;
   bool in_capture = false;
   uint32_t capture_failures = 0;
@@ -3131,6 +3141,17 @@ static LeanForm partition_form(const Plan& p, int partition_mode, int jit_mode, 
   return LEAN_PARTITIONED;
 }
 
+constexpr u64 kStageBytes = 64u << 10;  // results up to this size travel to page-locked memory behind the scan
+static u64 result_bytes(u64 gcap, uint32_t n_gwords, uint32_t n_keys) { return (gcap + 2) * n_gwords * 8 + (n_keys ? gcap * 8 : 0); }
+
+// The step form of a run, for the runtime and for llkv_gpu_debug_plan alike: true when the scan publishes its result itself
+// (LeanPlan::publish) and a repeated step is that one kernel.  It needs the lean plan in its per-row form, a result that fits
+// the stage, group keys that need no pass over the table on the device (hashed wide keys are verified there), one rank, and
+// a run that starts from the initial state (the kernel re-arms it).  Any other run is reset, scan and result copy.
+static bool step_publishes(bool per_row_lean, u64 bytes, uint32_t single_wide_key, int n_ranks, bool from_reset) {
+  return per_row_lean && bytes <= kStageBytes && single_wide_key != 2 && n_ranks == 1 && from_reset;
+}
+
 static int32_t lean_geometry(const LeanTune& tn, const Plan& p, uint64_t row_begin, uint64_t row_end, uint64_t hint, LeanPlan& lp, Geometry& g,
                              uint32_t* ctas_out) {
   memset(&lp, 0, sizeof(lp));
@@ -3528,6 +3549,11 @@ extern "C" int32_t llkv_gpu_debug_plan(const llkv_debug_column* cols, int32_t n_
     }
     lp.s.use_tile_list = (jit & 4) ? 1u : 0u;  // jit bit 2: the variant that walks a zone-map tile list
     text = lean_listing(lp, g, ctas);
+    // jit bit 4: a run that continues from the previous one (no reset in between)
+    const u64 gcap = cr.plan.n_keys ? group_table_cap(cardinality_hint) : 1;
+    text += step_publishes(form == LEAN_INTERPRETED, result_bytes(gcap, cr.plan.n_gwords, cr.plan.n_keys), cr.plan.single_wide_key, 1, !(jit & 16))
+                ? "step: one kernel, the scan publishes the result to page-locked memory and re-arms the state\n"
+                : "step: reset, scan, result copy\n";
     if (jit & 1) {
       std::vector<char> cubin;
       std::string log;
@@ -3661,8 +3687,8 @@ extern "C" int32_t llkv_gpu_agg_create(llkv_gpu_ctx* ctx, uint64_t table_id, con
   a->expr_mode = expr_mode;
   a->hint = cardinality_hint;
   memset(&a->info, 0, sizeof(a->info));
-  cudaError_t e = cudaMalloc((void**)&a->d_flags, 4);
-  if (e == cudaSuccess) e = cudaMemset(a->d_flags, 0, 4);
+  cudaError_t e = cudaMalloc((void**)&a->d_flags, 8);  // [status word, ticket of a publishing scan]
+  if (e == cudaSuccess) e = cudaMemset(a->d_flags, 0, 8);
   if (e == cudaSuccess) e = cudaMalloc((void**)&a->d_plan, sizeof(Plan));
   if (e == cudaSuccess) e = cudaHostAlloc((void**)&a->h_plan, sizeof(Plan), cudaHostAllocDefault);
   if (e == cudaSuccess) e = cudaHostAlloc((void**)&a->h_flags, 4, cudaHostAllocDefault);
@@ -3733,6 +3759,7 @@ extern "C" void llkv_gpu_agg_destroy(llkv_gpu_agg* a) {
   if (a->h_plan) cudaFreeHost(a->h_plan);
   if (a->h_flags) cudaFreeHost(a->h_flags);
   if (a->h_stage) cudaFreeHost(a->h_stage);
+  if (a->h_pub) cudaFreeHost(a->h_pub);
   delete a;
 }
 
@@ -3780,6 +3807,7 @@ static int32_t agg_backup(llkv_gpu_agg* a) {
 }
 static int32_t agg_restore(llkv_gpu_agg* a) {
   llkv_gpu_ctx* ctx = a->ctx;
+  a->armed = false;
   CUDA_TRY(cudaMemcpyAsync(a->gkeys, a->bk_keys, a->gcap * 8, cudaMemcpyDeviceToDevice, ctx->stream));
   CUDA_TRY(cudaMemcpyAsync(a->gwords, a->bk_words, (a->gcap + 2) * a->n_gwords * 8, cudaMemcpyDeviceToDevice, ctx->stream));
   return LLKV_OK;
@@ -3791,6 +3819,7 @@ static int32_t agg_grow_table(llkv_gpu_agg* a) {
   u64* old_keys = a->gkeys;
   u64* old_words = a->gwords;
   const u64 old_cap = a->gcap;
+  a->armed = false;
   a->gkeys = nullptr;
   a->gwords = nullptr;
   int32_t rc = agg_alloc_table(a, old_cap * 4);
@@ -4020,13 +4049,13 @@ static int32_t agg_queue_result_copy(llkv_gpu_agg* a) {
   CUDA_TRY(cudaMemcpyAsync(a->h_flags, a->d_flags, 4, cudaMemcpyDeviceToHost, ctx->stream));
   a->prefetched = false;
   const size_t wbytes = (size_t)(a->gcap + 2) * a->n_gwords * 8, kbytes = a->cr.plan.n_keys ? (size_t)a->gcap * 8 : 0;
-  if (wbytes + kbytes > (64u << 10)) return LLKV_OK;
+  if (wbytes + kbytes > kStageBytes) return LLKV_OK;
   if (a->h_stage_bytes < wbytes + kbytes) {
     if (a->h_stage) CUDA_TRY(cudaFreeHost(a->h_stage));
     a->h_stage = nullptr;
     a->h_stage_bytes = 0;
-    CUDA_TRY(cudaHostAlloc((void**)&a->h_stage, 64u << 10, cudaHostAllocDefault));
-    a->h_stage_bytes = 64u << 10;
+    CUDA_TRY(cudaHostAlloc((void**)&a->h_stage, kStageBytes, cudaHostAllocDefault));
+    a->h_stage_bytes = kStageBytes;
   }
   CUDA_TRY(cudaMemcpyAsync(a->h_stage, a->gwords, wbytes, cudaMemcpyDeviceToHost, ctx->stream));
   if (kbytes) CUDA_TRY(cudaMemcpyAsync(a->h_stage + wbytes, a->gkeys, kbytes, cudaMemcpyDeviceToHost, ctx->stream));
@@ -4047,6 +4076,7 @@ struct RunLaunches {
   FoldPlan fp;         // packed form: the partition_fold pass behind every scan launch
   uint32_t part_grid = 0;
   bool use_tile_list = false;
+  bool publish = false;  // step_publishes: the last launch publishes the result and re-arms the state
 };
 
 // Compiles the request and freezes the accumulator layout, unless the lean plan of the previous run still applies
@@ -4414,6 +4444,7 @@ static int32_t agg_run_launches(llkv_gpu_agg* a, uint64_t row_begin, uint64_t ro
   if (ctx->timing) CUDA_TRY(cudaEventRecord(ctx->ev0, ctx->stream));
   uint32_t launches = 0;
   a->info.used_jit_kernel = 0;
+  a->published = false;
   lean.tile_list = nullptr;
   lean.s.use_tile_list = r.use_tile_list ? 1u : 0u;
   const u64 list_n = r.use_tile_list ? a->h_tile_list.size() : 0;
@@ -4439,11 +4470,19 @@ static int32_t agg_run_launches(llkv_gpu_agg* a, uint64_t row_begin, uint64_t ro
     if (n_tiles == 0) break;
     const u64 grid = std::min<u64>(r.g.grid, n_tiles);
     if (!launches) a->info.grid = (uint32_t)grid;
+    const bool last = r.use_tile_list ? list_pos >= list_n : re >= row_end;
+    a->armed = false;
     if (a->cr.fast) {
       lean.row_begin = rb;
       lean.row_end = re;
       lean.first_tile = first_tile;
       lean.n_tiles = n_tiles;
+      if (r.publish && last) {
+        lean.publish = a->d_pub;
+        lean.ticket = a->d_flags + 1;
+        lean.gclass = a->d_gclass;
+        a->armed = a->published = true;
+      }
       bool jitted = false;
       if (partitioned) CUDA_TRY(cudaMemsetAsync(a->part_cursor, 0, kMaxPackedPartitions * 4, ctx->stream));
       if (r.use_jit) CUDA_TRY(jit_launch(ctx->device, lean, (int)r.lean_ctas, (uint32_t)grid, ctx->stream, &jitted, nullptr));
@@ -4471,8 +4510,9 @@ static int32_t agg_run_launches(llkv_gpu_agg* a, uint64_t row_begin, uint64_t ro
       CUDA_TRY(launch_scan(a->d_plan, a->cr.wide, (int)r.g.R, (uint32_t)grid, r.g.block, r.g.smem, ctx->stream));
     }
     ++launches;
-    if (r.use_tile_list ? list_pos >= list_n : re >= row_end) break;
+    if (last) break;
   }
+  lean.publish = nullptr;
   if (ctx->timing) CUDA_TRY(cudaEventRecord(ctx->ev1, ctx->stream));
   *launches_out = launches;
   return LLKV_OK;
@@ -4508,9 +4548,21 @@ static int32_t agg_launch(llkv_gpu_agg* a, const llkv_gpu_program* prog, int app
   a->cr.plan.exists_bits = exists_bits;
   if (a->cr.fast && (rc = agg_choose_form(a, row_begin, row_end, r))) return rc;
   if ((rc = agg_bind_state(a, handles))) return rc;
-  const bool need_backup = a->cr.can_narrow_fail || a->cr.plan.n_keys != 0;
+  // a run from the initial state needs no backup: a rerun starts again from the initial state
+  const bool from_reset = a->armed;
+  const bool need_backup = !from_reset && (a->cr.can_narrow_fail || a->cr.plan.n_keys != 0);
   if (need_backup && (rc = agg_backup(a))) return rc;
   a->pending.has_backup = need_backup;
+  a->pending.from_reset = from_reset;
+  r.publish = step_publishes(a->cr.fast && a->lean.s.partition == 0, result_bytes(a->gcap, a->n_gwords, a->cr.plan.n_keys), a->cr.plan.single_wide_key,
+                             ctx->n_ranks, from_reset);
+  if (r.publish && !a->h_pub) {
+    if (a->in_capture) r.publish = false;  // (no allocation inside a stream capture: this step keeps the copy)
+    else {
+      CUDA_TRY(cudaHostAlloc((void**)&a->h_pub, 8 + kStageBytes, cudaHostAllocMapped));
+      CUDA_TRY(cudaHostGetDevicePointer((void**)&a->d_pub, a->h_pub, 0));
+    }
+  }
   // thread-private partial sums stay exact while a thread folds a bounded number of rows per launch: split very long scans
   // (general interpreter: < 2^15 rows per thread; lean kernel: 2^kLeanRowsPerThreadLog2 rows per consumer thread, and
   // launch-relative row indices must fit 32 bits)
@@ -4521,7 +4573,7 @@ static int32_t agg_launch(llkv_gpu_agg* a, const llkv_gpu_program* prog, int app
   if ((rc = agg_tile_list(a, sig, handles, table_rows, row_begin, row_end, &r.use_tile_list))) return rc;
   uint32_t launches = 0;
   if ((rc = agg_run_launches(a, row_begin, row_end, r, &launches))) return rc;
-  if (!a->skip_scan_copy && (rc = agg_queue_result_copy(a))) return rc;
+  if (!a->published && !a->skip_scan_copy && (rc = agg_queue_result_copy(a))) return rc;
   a->info.rows = row_end - row_begin;
   a->info.kernel_launches = launches;
   a->info.used_wide_path = a->cr.wide ? 1 : 0;
@@ -4549,12 +4601,31 @@ static int32_t agg_fail(llkv_gpu_agg* a, int32_t code, const char* fmt, ...) {
 
 // llkv_gpu_agg_reset only marks the state; the status word and the table are cleared here, in stream order, right before
 // whatever uses them next (so a reset and the scan that follows it are one run of launches — and one captured graph)
-static int32_t agg_apply_reset(llkv_gpu_agg* a) {
-  if (!a->reset_pending) return LLKV_OK;
+// Puts the status word and the table back to their initial values, in stream order (nothing while the state is armed)
+static int32_t agg_rearm(llkv_gpu_agg* a) {
+  if (a->armed) return LLKV_OK;
   llkv_gpu_ctx* ctx = a->ctx;
-  a->reset_pending = false;
   CUDA_TRY(cudaMemsetAsync(a->d_flags, 0, 4, ctx->stream));
   if (a->frozen) CUDA_TRY(launch_init_table(a->gkeys, a->gwords, a->gcap + 2, a->n_gwords, a->d_gclass, ctx->stream));
+  a->armed = a->frozen;
+  return LLKV_OK;
+}
+static int32_t agg_apply_reset(llkv_gpu_agg* a) {
+  if (!a->reset_pending) return LLKV_OK;
+  a->reset_pending = false;
+  a->published = false;  // (the published result is dropped; the scan that published it re-armed the state)
+  return agg_rearm(a);
+}
+
+// Something continues from the published result (a run without a reset, a merge): the table goes back onto the device
+static int32_t agg_unpublish(llkv_gpu_agg* a) {
+  if (!a->published) return LLKV_OK;
+  llkv_gpu_ctx* ctx = a->ctx;
+  a->published = false;
+  a->armed = false;
+  const u64 n_words = (a->gcap + 2) * a->n_gwords;
+  CUDA_TRY(cudaMemcpyAsync(a->gwords, a->h_pub + 1, n_words * 8, cudaMemcpyHostToDevice, ctx->stream));
+  if (a->cr.plan.n_keys) CUDA_TRY(cudaMemcpyAsync(a->gkeys, a->h_pub + 1 + n_words, a->gcap * 8, cudaMemcpyHostToDevice, ctx->stream));
   return LLKV_OK;
 }
 
@@ -4576,9 +4647,10 @@ static int32_t agg_resolve(llkv_gpu_agg* a) {
       if (cudaEventElapsedTime(&ms, ctx->ev2, ctx->ev3) == cudaSuccess) a->info.last_merge_ms = ms;
       else cudaGetLastError();
     }
-    const uint32_t flags = *a->h_flags;
+    const uint32_t flags = a->published ? (uint32_t)a->h_pub[0] : *a->h_flags;
     if (flags == 0) break;
     a->prefetched = false;  // the run is repeated or failed: what travelled behind it is not the result
+    a->published = false;   // (the scan that published it re-armed the state)
     CUDA_TRY(cudaMemsetAsync(a->d_flags, 0, 4, ctx->stream));
     *a->h_flags = 0;
     const bool narrow_fail = (flags & FLAG_NARROW_FAIL) && !a->pending.wide;
@@ -4622,8 +4694,8 @@ static int32_t agg_resolve(llkv_gpu_agg* a) {
       continue;
     }
     if (narrow_fail || table_full) {
-      if (!a->pending.has_backup) return agg_fail(a, LLKV_ERR_INTERNAL, "device asked for a rerun without a saved state");
-      int32_t rc = agg_restore(a);
+      if (!a->pending.from_reset && !a->pending.has_backup) return agg_fail(a, LLKV_ERR_INTERNAL, "device asked for a rerun without a saved state");
+      int32_t rc = a->pending.from_reset ? agg_rearm(a) : agg_restore(a);
       if (rc) return rc;
       if (table_full && (rc = agg_grow_table(a))) return rc;
       if (narrow_fail) a->pending.wide = true;
@@ -4680,6 +4752,7 @@ static int32_t agg_run_impl(llkv_gpu_agg* a, const llkv_gpu_program* prog, int32
   if (a->err_code) return set_error(a->err_code, "%s", a->err_msg.c_str());
   int32_t rc = agg_resolve(a);
   if (rc) return rc;
+  if ((rc = agg_unpublish(a))) return rc;
   a->pending.has_prog = prog != nullptr;
   if (prog && a->pending.prog.serial != prog->serial) {
     a->pending.prog.ops = prog->ops;
@@ -4987,7 +5060,10 @@ static int32_t agg_collect(llkv_gpu_agg* a, std::vector<u64>& hk, std::vector<u6
   hk.resize(a->gcap);
   hw.resize(rows * a->n_gwords);
   const size_t wbytes = hw.size() * 8, kbytes = a->cr.plan.n_keys ? hk.size() * 8 : 0;
-  if (a->prefetched && a->h_stage_bytes >= wbytes + kbytes) {  // already on its way (agg_queue_result_copy)
+  if (a->published) {  // the scan put it there (agg_resolve waited for it)
+    memcpy(hw.data(), a->h_pub + 1, wbytes);
+    if (kbytes) memcpy(hk.data(), a->h_pub + 1 + hw.size(), kbytes);
+  } else if (a->prefetched && a->h_stage_bytes >= wbytes + kbytes) {  // already on its way (agg_queue_result_copy)
     // usually complete: agg_resolve waited for the run.  Not when the copy was queued with no run pending (a merge behind
     // a run that had to be settled first).
     if (a->stage_ev_valid) CUDA_TRY(cudaEventSynchronize(a->stage_ev));
@@ -5422,6 +5498,10 @@ static int32_t agg_merge_impl(llkv_gpu_agg* a) {
     return set_error(LLKV_ERR_INVALID_ARGUMENT, "GROUP BY keys wider than 64 bits do not merge across GPUs: a group's key values are read from the shard that holds its first row");
   int32_t rc;
   if (!a->pending.active && (rc = agg_apply_reset(a))) return rc;
+  if (ctx->nccl_comm && ctx->n_ranks > 1) {  // the merge works on the table on the device
+    if (a->published && ((rc = agg_resolve(a)) || (rc = agg_unpublish(a)))) return rc;
+    a->armed = false;
+  }
   a->prefetched = false;  // the merge rewrites the table
   const int N = ctx->n_ranks;
   const int nccl_u64 = 5 /* ncclUint64 */, nccl_max = 2 /* ncclMax */;
@@ -5582,7 +5662,7 @@ extern "C" int32_t llkv_gpu_agg_execute(llkv_gpu_agg* a, const llkv_gpu_program*
     key = fnv1a(key, parts, sizeof(parts));
     if (!key) key = 1;
   }
-  if (a->graph_exec && a->graph_key == key && prev_clean) {
+  if (a->graph_exec && a->graph_key == key && prev_clean && (!a->graph_from_armed || a->armed)) {
     const PendingRun& gp = a->graph_pending;  // (the program copy of the captured step is still in a->pending.prog)
     a->pending.has_prog = gp.has_prog;
     a->pending.apply_mvcc = gp.apply_mvcc;
@@ -5597,6 +5677,8 @@ extern "C" int32_t llkv_gpu_agg_execute(llkv_gpu_agg* a, const llkv_gpu_program*
     CUDA_TRY(cudaGraphLaunch(a->graph_exec, ctx->stream));
     ++a->info.graph_replays;
     a->prefetched = a->graph_prefetched;
+    a->published = a->graph_published;
+    a->armed = a->graph_armed_after;
     a->stage_ev_valid = false;
     a->pending.active = true;
     a->info.kernel_launches = a->graph_launches;
@@ -5615,6 +5697,7 @@ extern "C" int32_t llkv_gpu_agg_execute(llkv_gpu_agg* a, const llkv_gpu_program*
       a->graph_key = 0;
     }
     a->in_capture = true;
+    const bool armed_before = a->armed;
     cudaError_t e = cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal);
     int32_t rc = LLKV_OK;
     if (e == cudaSuccess) {
@@ -5638,6 +5721,9 @@ extern "C" int32_t llkv_gpu_agg_execute(llkv_gpu_agg* a, const llkv_gpu_program*
       a->graph_pending = a->pending;
       a->graph_pending.prog = llkv_gpu_program();
       a->graph_prefetched = a->prefetched;
+      a->graph_from_armed = armed_before;
+      a->graph_published = a->published;
+      a->graph_armed_after = a->armed;
       a->graph_launches = a->info.kernel_launches;
       a->stage_ev_valid = false;
       return LLKV_OK;
@@ -5652,6 +5738,8 @@ extern "C" int32_t llkv_gpu_agg_execute(llkv_gpu_agg* a, const llkv_gpu_program*
     ++a->capture_failures;
     a->pending.active = false;
     a->prefetched = false;
+    a->published = false;
+    a->armed = false;  // (the captured resets never ran)
     a->reset_pending = true;
     cudaStreamSynchronize(ctx->stream);
     cudaGetLastError();

@@ -353,6 +353,12 @@ struct LeanPlan {
   // zone-map pruning: when set, the launch visits tiles tile_list[0 .. n_tiles) (ascending, >= first_tile) instead of
   // first_tile .. first_tile + n_tiles: the host dropped the tiles whose zones no conjunct range leaf can match
   const uint32_t* tile_list;
+  // publishing step (set on the last launch of a run that starts from the initial state): the CTA that finishes last copies
+  // the status word, the (gcap + 2) x n_gwords words and, grouped, the gcap keys to publish[0], publish[1 ..] (page-locked
+  // host memory mapped into the device) and puts the state back to its initial value.  Null: the state stays as it is.
+  unsigned long long* publish;
+  uint32_t* ticket;        // CTAs of the launch done so far (0 between launches)
+  const uint8_t* gclass;   // WordClass of each of the n_gwords words of a group row
 };
 constexpr uint32_t kZoneRows = 4096;  // rows per zone-map entry (= the reference's chunk of Decimal128 / Date32 rows, slicing.rs:155-166)
 

@@ -952,10 +952,7 @@ __global__ void init_table_kernel(u64* keys, u64* words, u64 rows, uint32_t n_gw
   const u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x;
   const u64 total = rows * n_gwords;
   if (keys && i + 2 < rows) keys[i] = kEmptyKey;  // `rows` counts the two spare rows (reserved key value, NULL key), which have no key slot
-  for (u64 j = i; j < total; j += (u64)gridDim.x * blockDim.x) {
-    const uint8_t c = word_class_dev[j % n_gwords];
-    words[j] = (c == WC_MIN || c == WC_MIN128 || c == WC_PAIR_LO_MIN) ? ~0ull : 0ull;
-  }
+  for (u64 j = i; j < total; j += (u64)gridDim.x * blockDim.x) words[j] = gword_initial(word_class_dev[j % n_gwords]);
 }
 
 // merge kernel for gathered partial tables (multi-GPU GROUP BY): rows of `src` are folded into the local table

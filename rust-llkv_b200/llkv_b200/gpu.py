@@ -630,9 +630,10 @@ def merge_partial_results(parts, rules):
 def debug_plan(table: HostTable, expr: Optional[Expr], specs: Sequence[AggregateSpec], snapshot: Optional[Snapshot] = None,
                group_by: Sequence[int] = (), expr_mode: Optional[int] = None, cardinality_hint: int = 0, block_threads: int = 0,
                rows_per_thread: int = 0, stages: int = 0, ctas_per_sm: int = 0, jit: bool = False, cubin_path: Optional[str] = None,
-               partition: bool = False, tile_list: bool = False, packed: bool = False) -> str:
+               partition: bool = False, tile_list: bool = False, packed: bool = False, continues: bool = False) -> str:
     """llkv_gpu_debug_plan: compiles the plan against the host table's column statistics (no GPU needed) and returns the
-    listing of the lean program; with jit=True the lean kernel is also specialised with NVRTC."""
+    listing of the lean program; with jit=True the lean kernel is also specialised with NVRTC.  continues=True: the step
+    form of a run that follows another run without a reset."""
     lib = load()
     cols = []
     host_cols = list(table.columns.values())
@@ -684,7 +685,7 @@ def debug_plan(table: HostTable, expr: Optional[Expr], specs: Sequence[Aggregate
         out = C.create_string_buffer(1 << 16)
         _check(lib.llkv_gpu_debug_plan(arr, len(host_cols), prog, created, deleted, snapshot.txn_id if snapshot else 0,
                                        snapshot.snapshot_id if snapshot else 0, aggs, n_aggs, anodes, n_anodes, keys, len(group_by), expr_mode,
-                                       cardinality_hint, block_threads, rows_per_thread, stages, ctas_per_sm, int(jit) | (2 if partition or packed else 0) | (4 if tile_list else 0) | (8 if packed else 0),
+                                       cardinality_hint, block_threads, rows_per_thread, stages, ctas_per_sm, int(jit) | (2 if partition or packed else 0) | (4 if tile_list else 0) | (8 if packed else 0) | (16 if continues else 0),
                                        cubin_path.encode() if cubin_path else None, out, len(out)))
         return out.value.decode()
     finally:
