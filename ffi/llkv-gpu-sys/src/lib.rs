@@ -204,6 +204,7 @@ pub struct llkv_run_info {
     pub merged_p2p: u32,
     pub last_merge_ms: f32,
     pub packed_tuples: u32,
+    pub published_steps: u32,
 }
 
 #[repr(C)]

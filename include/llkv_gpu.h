@@ -245,6 +245,8 @@ typedef struct llkv_run_info {
   float last_merge_ms;          /* device time of that merge kernel, waiting for the slowest peer included (timing enabled) */
   uint32_t packed_tuples;       /* partitioned run in its packed form (64-bit tuples, partitions aggregated in shared memory):
                                    1 = partitions are hash ranges, 2 = key ranges (dense integer keys); 0 = first form / not partitioned */
+  uint32_t published_steps;     /* steps of this aggregate whose scan published the result to page-locked memory and re-armed
+                                   the state (a repeated step that is one kernel), replays included */
 } llkv_run_info;
 
 typedef struct llkv_gpu_ctx llkv_gpu_ctx;

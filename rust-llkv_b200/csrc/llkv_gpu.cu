@@ -3776,16 +3776,32 @@ static int32_t agg_alloc_table(llkv_gpu_agg* a, u64 gcap) {
 
 static int32_t agg_freeze_layout(llkv_gpu_agg* a, const CompileResult& cr) {
   const Plan& p = cr.plan;
+  u64 cap = p.n_keys ? group_table_cap(a->hint) : 1;
   if (a->frozen) {
-    if (p.n_gwords != a->n_gwords || memcmp(p.gword_class, a->gclass.data(), a->n_gwords) != 0)
-      return set_error(LLKV_ERR_INTERNAL, "accumulator layout changed between runs (column types changed?)");
-    return LLKV_OK;
+    if (p.n_gwords == a->n_gwords && memcmp(p.gword_class, a->gclass.data(), a->n_gwords) == 0) return LLKV_OK;
+    // The layout follows facts of the request as well as the aggregates: a COUNT over a column that cannot hold NULLs is
+    // the row count and has no word of its own, and appended or deleted rows can give a column NULLs.  A state that holds
+    // nothing yet (armed: a reset or a new step) takes the new layout; a run cannot continue a state of the old one.
+    if (!a->armed || a->in_capture)
+      return set_error(LLKV_ERR_INVALID_ARGUMENT, "accumulator layout changed since the aggregate's state was started (a column gained "
+                       "NULLs?): reset the aggregate before running over the changed table");
+    llkv_gpu_ctx* ctx = a->ctx;
+    CUDA_TRY(cudaStreamSynchronize(ctx->stream));  // (queued launches may still read the old table or classes)
+    CUDA_TRY(cudaFree(a->gkeys));
+    CUDA_TRY(cudaFree(a->gwords));
+    CUDA_TRY(cudaFree(a->d_gclass));
+    if (a->bk_keys) CUDA_TRY(cudaFree(a->bk_keys));
+    if (a->bk_words) CUDA_TRY(cudaFree(a->bk_words));
+    a->gkeys = a->gwords = a->bk_keys = a->bk_words = nullptr;
+    a->d_gclass = nullptr;
+    a->bk_cap = 0;
+    cap = a->gcap;  // (a table grown for this aggregate's groups keeps its size)
   }
   a->n_gwords = p.n_gwords;
   a->gclass.assign(p.gword_class, p.gword_class + p.n_gwords);
   CUDA_TRY(cudaMalloc((void**)&a->d_gclass, a->n_gwords ? a->n_gwords : 1));
   CUDA_TRY(cudaMemcpy(a->d_gclass, a->gclass.data(), a->n_gwords, cudaMemcpyHostToDevice));
-  int32_t rc = agg_alloc_table(a, p.n_keys ? group_table_cap(a->hint) : 1);
+  int32_t rc = agg_alloc_table(a, cap);
   if (rc) return rc;
   a->frozen = true;
   return LLKV_OK;
@@ -4482,6 +4498,7 @@ static int32_t agg_run_launches(llkv_gpu_agg* a, uint64_t row_begin, uint64_t ro
         lean.ticket = a->d_flags + 1;
         lean.gclass = a->d_gclass;
         a->armed = a->published = true;
+        ++a->info.published_steps;
       }
       bool jitted = false;
       if (partitioned) CUDA_TRY(cudaMemsetAsync(a->part_cursor, 0, kMaxPackedPartitions * 4, ctx->stream));
@@ -5676,6 +5693,7 @@ extern "C" int32_t llkv_gpu_agg_execute(llkv_gpu_agg* a, const llkv_gpu_program*
     a->reset_pending = false;  // part of the graph
     CUDA_TRY(cudaGraphLaunch(a->graph_exec, ctx->stream));
     ++a->info.graph_replays;
+    if (a->graph_published) ++a->info.published_steps;
     a->prefetched = a->graph_prefetched;
     a->published = a->graph_published;
     a->armed = a->graph_armed_after;
@@ -5698,6 +5716,7 @@ extern "C" int32_t llkv_gpu_agg_execute(llkv_gpu_agg* a, const llkv_gpu_program*
     }
     a->in_capture = true;
     const bool armed_before = a->armed;
+    const uint32_t published_before = a->info.published_steps;
     cudaError_t e = cudaStreamBeginCapture(ctx->stream, cudaStreamCaptureModeThreadLocal);
     int32_t rc = LLKV_OK;
     if (e == cudaSuccess) {
@@ -5739,6 +5758,7 @@ extern "C" int32_t llkv_gpu_agg_execute(llkv_gpu_agg* a, const llkv_gpu_program*
     a->pending.active = false;
     a->prefetched = false;
     a->published = false;
+    a->info.published_steps = published_before;  // (the captured scan never ran; the plain run below counts the step)
     a->armed = false;  // (the captured resets never ran)
     a->reset_pending = true;
     cudaStreamSynchronize(ctx->stream);

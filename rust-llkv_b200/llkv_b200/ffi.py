@@ -93,7 +93,8 @@ class RunInfo(C.Structure):
                 ("grid", C.c_uint32), ("block", C.c_uint32), ("rows_per_tile", C.c_uint32), ("stages", C.c_uint32),
                 ("smem_bytes", C.c_uint32), ("fast_groups", C.c_uint32), ("last_kernel_ms", C.c_float),
                 ("used_fast_kernel", C.c_uint32), ("used_jit_kernel", C.c_uint32), ("partitions", C.c_uint32), ("tiles_pruned", C.c_uint32),
-                ("graph_replays", C.c_uint32), ("merged_p2p", C.c_uint32), ("last_merge_ms", C.c_float), ("packed_tuples", C.c_uint32)]
+                ("graph_replays", C.c_uint32), ("merged_p2p", C.c_uint32), ("last_merge_ms", C.c_float), ("packed_tuples", C.c_uint32),
+                ("published_steps", C.c_uint32)]
 
 
 class DebugColumn(C.Structure):
